@@ -12,6 +12,9 @@ Prints ONE JSON line (rank 0).  A "step" is the reconstruction of one frame (bat
               SAME frame at full size on the host cores (rank 0, N = 1)
  parity       per-level rel-L2 / max-abs / log-det error of the bf16 AND fp16 engines against that CPU run of the same frame
  extra        module-API frames/s, forward NLL (eager + CUDA graph), DP training step (configs[3]), 1024-frame stream (configs[4])
+
+--dump-outputs DIR writes the volume the last timed step reconstructed (rank 0) to DIR/volume.npy, so that two builds can be
+compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -32,6 +35,8 @@ UNIT = "frames/s"
 PUBLISHED_FPS = 1.0 / 0.16          # reference README.md:29 "around 0.16 seconds per frame", hardware not stated
 # SURVEY.md 8(d): algorithmic conv flops (2*MAC, true channel counts) of one full inverse frame
 FRAME_FLOP = 4.3971e12
+# --dump-outputs: an array larger than this many elements is stored as a fixed sample (32 MiB in float32)
+DUMP_MAX_ELEMS = 8 << 20
 
 
 def conv_flops_per_frame(cfg):
@@ -204,6 +209,20 @@ def bind_to_gpu_numa_node(index: int):
         return None, why + f"; sysfs lookup failed ({type(ex).__name__})"
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor of ``arrays`` as ``out_dir/<name>.npy`` in float32.  A tensor of more than DUMP_MAX_ELEMS elements is
+    stored as the 1-D sample of its flattened values at DUMP_MAX_ELEMS positions drawn without replacement by a generator seeded
+    with 0, in increasing order: the positions depend on the shape only, so dumps of two builds compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > DUMP_MAX_ELEMS:
+            pos = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            a = a.reshape(-1)[pos]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 def pctl(vals, q):
     vals = sorted(vals)
     return vals[min(len(vals) - 1, int(round(q * (len(vals) - 1))))]
@@ -230,7 +249,12 @@ def main():
                          "default autocast, CWFA.py:845; the other dtype is measured too and reported in extra)")
     ap.add_argument("--inflight", type=int, default=2, help="graph instances (frames) in flight per GPU")
     ap.add_argument("--e2e-inflight", type=int, default=2, help="frames in flight in the host-buffer streaming measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the volume the last of them reconstructed (rank 0) to DIR/volume.npy "
+                         "(float32; a fixed seeded sample of its elements when it is larger than 32 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(side=args.side, depths=args.depths, steps=args.down_steps)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -312,11 +336,13 @@ def main():
     outs_dev = [torch.empty((1, args.depths, args.side, args.side), device=dev, dtype=torch.float32) for _ in range(2)]
 
     def run_frames(k):
+        """Reconstructs k frames; returns the volume of the last one."""
         if streamer is None:
             for i in range(k):
-                eng.reconstruct(views_dev[i % n_rot], mvs_dev)
-        else:
-            streamer.run([views_dev[i % n_rot] for i in range(k)], [outs_dev[i % 2] for i in range(k)])
+                last = eng.reconstruct(views_dev[i % n_rot], mvs_dev)
+            return last
+        streamer.run([views_dev[i % n_rot] for i in range(k)], [outs_dev[i % 2] for i in range(k)])
+        return outs_dev[(k - 1) % 2]
 
     run_frames(max(3, args.warmup))
     barrier()
@@ -326,10 +352,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    run_frames(args.steps)
+    last_volume = run_frames(args.steps)
     e1.record()
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"volume": last_volume})
+    del last_volume
     # single-stream, one-graph-at-a-time latency of a frame (reported next to the throughput)
     if streamer is not None:
         l0, l1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
