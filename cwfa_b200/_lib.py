@@ -41,6 +41,7 @@ _SIGS = {
     "cwfa_tc_kc": [i32],
     "cwfa_tc_pack_weights": [vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp],
     "cwfa_conv_tc": [vp, vp, vp, vp, vp, vp] + [i32] * 14 + [vp],
+    "cwfa_conv_tc_plan": [i32] * 17 + [vp],
     "cwfa_conv_tc_bn": [vp, vp, vp, vp, vp] + [i32] * 12 + [vp, vp],
     "cwfa_bn_partial_finalize": [vp, i32, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp, vp],
     "cwfa_resblock_tc": [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp],
@@ -160,7 +161,7 @@ class CwfaError(RuntimeError):
 # kernel launches issued per C-ABI call (for bench.py's "gpu_launches" claim)
 _LAUNCHES = {"cwfa_bn_partial_finalize": 2, "cwfa_affine": 2, "cwfa_channel_stats_f32": 2, "cwfa_layernorm_chw_f32": 2, "cwfa_c8_channel_stats": 2, "cwfa_c8_layernorm": 2, "cwfa_conv2d_wgrad_f32": 2, "cwfa_wgrad_tc": 2, "cwfa_prelu_bwd_f32": 2, "cwfa_stencil3d_wgrad_f32": 2,
              "cwfa_reduce_workspace_blocks": 0, "cwfa_channel_dot_workspace_blocks": 0, "cwfa_channel_dot_stats_f32": 2, "cwfa_ln_bwd_stats_f32": 2, "cwfa_stencil3d_wgrad_workspace_floats": 0,
-             "cwfa_tc_set_debug_buffer": 0, "cwfa_resblock_set_debug_buffer": 0, "cwfa_device_check": 0, "cwfa_conv_tc_coupling_tiles": 0, "cwfa_coupling_tc_tiles": 0}
+             "cwfa_tc_set_debug_buffer": 0, "cwfa_resblock_set_debug_buffer": 0, "cwfa_device_check": 0, "cwfa_conv_tc_coupling_tiles": 0, "cwfa_coupling_tc_tiles": 0, "cwfa_conv_tc_plan": 0}
 launch_count = 0
 launch_hist = {}
 

@@ -1070,32 +1070,41 @@ struct CouplingArgs {
     int ch, axis, inverse; float kk, tscale;
 };
 
-static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* bias, const float* slope,
-                          const void* res, void* out, int N, int H, int W, int Cin_p, int Cout, int Cout_p, int KH,
-                          int KW, int BN, int MB, int act, int res_mode, int out_mode, int is_bf16, void* stream,
-                          const CouplingArgs* cpl, float* stats = nullptr) {
+// The 26 compiled variants, indexed by the plan's kernel index:
+//   0-11  ring path, (fp16 | bf16) x (generic | WIDE) x epilogue (generic, lean none, lean PReLU);
+//   12-19 fused coupling epilogue, (fp16 | bf16) x (fwd, inv, fwd + external shift, inv + external shift);
+//   20-25 resident weights, (fp16 | bf16) x epilogue (generic, lean none, lean PReLU).
+typedef void (*ConvTcKernel)(const CUtensorMap, const TcParams);
+static const ConvTcKernel kConvTcKernels[26] = {
+    conv_tc_kernel<false, 0, false, 0>, conv_tc_kernel<false, 0, false, 1>, conv_tc_kernel<false, 0, false, 2>,
+    conv_tc_kernel<false, 0, true, 0>, conv_tc_kernel<false, 0, true, 1>, conv_tc_kernel<false, 0, true, 2>,
+    conv_tc_kernel<true, 0, false, 0>, conv_tc_kernel<true, 0, false, 1>, conv_tc_kernel<true, 0, false, 2>,
+    conv_tc_kernel<true, 0, true, 0>, conv_tc_kernel<true, 0, true, 1>, conv_tc_kernel<true, 0, true, 2>,
+    conv_tc_kernel<false, 1, false, 0>, conv_tc_kernel<false, 2, false, 0>, conv_tc_kernel<false, 3, false, 0>, conv_tc_kernel<false, 4, false, 0>,
+    conv_tc_kernel<true, 1, false, 0>, conv_tc_kernel<true, 2, false, 0>, conv_tc_kernel<true, 3, false, 0>, conv_tc_kernel<true, 4, false, 0>,
+    conv_tc_kernel<false, 0, false, 0, true>, conv_tc_kernel<false, 0, false, 1, true>, conv_tc_kernel<false, 0, false, 2, true>,
+    conv_tc_kernel<true, 0, false, 0, true>, conv_tc_kernel<true, 0, false, 1, true>, conv_tc_kernel<true, 0, false, 2, true>};
+
+struct TcPlan { int ki, wide; int64_t grid; size_t smem; };
+
+// Every decision of a conv_tc launch that depends on the shapes alone: validation, tile geometry, the shared-memory plan, the
+// kernel variant and the grid.  Fills the geometry fields of p.  conv_tc_launch and cwfa_conv_tc_plan both call it, so the plan
+// a caller queries is the plan the launch uses.  cplmode: -1 plain convolution, else the fused coupling epilogue (0 fwd, 1 inv,
+// 2 fwd + external shift, 3 inv + external shift).
+static int conv_tc_plan(TcParams& p, TcPlan& pl, int N, int H, int W, int Cin_p, int Cout_p, int KH, int KW, int BN, int MB, int act,
+                        int res_mode, int out_mode, int is_bf16, bool has_slope, bool stats, int cplmode) {
     const int KC = pick_kc(Cin_p);
     if (N <= 0 || H <= 0 || W <= 0 || !KC || (Cin_p % 16) || (out_mode != 2 && (Cout_p % BN)) || (BN % 16) || BN < 16 || BN > 256 ||
         (MB != 1 && MB != 2) || MB * BN > 512 || !(KH & 1) || !(KW & 1) || KH > 7 || KW > 7 || out_mode < 0 ||
-        out_mode > 3 || (out_mode == 2 && (KH != 1 || KW != 1 || (BN % 32) || (2 * Cout_p) % BN)) || (out_mode == 3 && (!cpl || BN != Cout_p))) {
+        out_mode > 3 || (out_mode == 2 && (KH != 1 || KW != 1 || (BN % 32) || (2 * Cout_p) % BN)) || (out_mode == 3 && (cplmode < 0 || BN != Cout_p))) {
         set_error("conv_tc: unsupported configuration (Cin_p=%d Cout_p=%d BN=%d MB=%d K=%dx%d)", Cin_p, Cout_p, BN, MB, KH, KW);
         return CWFA_EINVAL;
     }
-    if (res_mode != 0 && !res) { set_error("conv_tc: res_mode set but res is NULL"); return CWFA_EINVAL; }
     if (out_mode != 1 && out_mode != 3 && (int64_t)H * W * 2 * Cout_p * (out_mode == 2 ? 4 : 1) >= (int64_t)1 << 32) {
         set_error("conv_tc: one output sample must stay below 4 GiB (32-bit in-sample offsets)");
         return CWFA_EINVAL;
     }
-    if ((reinterpret_cast<uintptr_t>(x_c8) & 15) || (reinterpret_cast<uintptr_t>(w_packed) & 15) ||
-        (out_mode != 3 && (reinterpret_cast<uintptr_t>(out) & 15))) {
-        set_error("conv_tc: pointers must be 16-byte aligned");
-        return CWFA_EINVAL;
-    }
-    EncodeTiledFn encode = get_encode();
-    if (!encode) { set_error("conv_tc: cuTensorMapEncodeTiled not available"); return CWFA_ECUDA; }
-
-    TcParams p{};
-    p.N = N; p.H = H; p.W = W; p.Cout = Cout; p.Cout_p = Cout_p; p.KH = KH; p.KW = KW;
+    p.N = N; p.H = H; p.W = W; p.Cout_p = Cout_p; p.KH = KH; p.KW = KW;
     p.MB = MB; p.BN = BN;
     p.tiles_x = ceil_div(W, 8 * MB);
     p.tiles_y = ceil_div(H, 16);
@@ -1135,7 +1144,7 @@ static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* b
         // 1x1 convolutions gain nothing (one tap per item either way).  The A ring stays at two stages: a deeper ring measured
         // +-0 for the small convs, and filling the 113 KB budget pushes the SM's shared-memory carve-out to its maximum, which
         // costs the epilogues their L1 (64 -> 64 1x1 + GELU + residual: 33.9 -> 41.9 us; level-0 training step +2.4 %).
-        if (nblks == 1 && KH * KW > 1 && stats == nullptr && out_mode != 3 && MB * BN <= 256 && (uint64_t)hdr + 2ull * p.a_stride + (uint64_t)total_b * p.b_bytes <= budget &&
+        if (nblks == 1 && KH * KW > 1 && !stats && out_mode != 3 && MB * BN <= 256 && (uint64_t)hdr + 2ull * p.a_stride + (uint64_t)total_b * p.b_bytes <= budget &&
             (uint64_t)total_b * p.b_bytes < (1u << 20)) {
             p.b_resident = 1;
             p.a_stages = 2;
@@ -1146,6 +1155,50 @@ static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* b
     if (fixed + bs * p.b_bytes > budget_max) { set_error("conv_tc: tile does not fit shared memory"); return CWFA_EINVAL; }
     p.b_stages = bs;
     p.act = act; p.res_mode = res_mode; p.out_mode = out_mode; p.is_bf16 = is_bf16;
+    pl.smem = fixed + (size_t)bs * p.b_bytes;
+
+    pl.wide = out_mode != 3 && MB * BN > 256;      // > 256 TMEM columns: one CTA per SM anyway
+    // lean epilogue variants: C8 output, no residual, activation none / PReLU
+    const int fast = (out_mode == 0 && res_mode == 0) ? (act == CWFA_ACT_NONE ? 1 : (act == CWFA_ACT_PRELU && has_slope) ? 2 : 0) : 0;
+    if (stats && (fast == 0 || !pl.wide)) {
+        set_error("conv_tc: fused BatchNorm statistics need the lean epilogue of the wide kernel (C8 output, no residual, act none / PReLU, MB * BN > 256)");
+        return CWFA_EINVAL;
+    }
+    if (out_mode == 3) pl.ki = 12 + (is_bf16 ? 4 : 0) + cplmode;
+    else if (p.b_resident) pl.ki = 20 + (is_bf16 ? 3 : 0) + fast;
+    else pl.ki = (is_bf16 ? 6 : 0) + (pl.wide ? 3 : 0) + fast;
+    const int64_t items = (int64_t)p.tiles_x * p.tiles_y * N * ((out_mode == 2 ? 4 : 1) * Cout_p / BN);
+    if (items > 0x7fffffff) { set_error("conv_tc: too many tiles"); return CWFA_EINVAL; }
+    p.total_items = (int)items;
+    // Persistent grid: each CTA walks items blockIdx.x, +grid, ... so TMEM allocation, barrier set-up and the
+    // first-operand TMA latency are paid once per CTA, and (MB*BN <= 128) two accumulator buffers overlap the
+    // MMAs of the next item with this item's epilogue.  The coupling variants keep one item per CTA.
+    p.acc_bufs = (out_mode != 3 && MB * BN <= 128) ? 2 : 1;
+    const int occ = (pl.wide || pl.smem > 113 * 1024) ? 1 : 2;
+    pl.grid = out_mode == 3 ? items : (items < (int64_t)kNumSMs * occ ? items : (int64_t)kNumSMs * occ);
+    return CWFA_OK;
+}
+
+static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* bias, const float* slope,
+                          const void* res, void* out, int N, int H, int W, int Cin_p, int Cout, int Cout_p, int KH,
+                          int KW, int BN, int MB, int act, int res_mode, int out_mode, int is_bf16, void* stream,
+                          const CouplingArgs* cpl, float* stats = nullptr) {
+    TcParams p{};
+    TcPlan pl{};
+    const int cplmode = cpl ? (cpl->t ? 2 : 0) + (cpl->inverse ? 1 : 0) : -1;
+    int rc = conv_tc_plan(p, pl, N, H, W, Cin_p, Cout_p, KH, KW, BN, MB, act, res_mode, out_mode, is_bf16, slope != nullptr,
+                          stats != nullptr, cplmode);
+    if (rc) return rc;
+    if (res_mode != 0 && !res) { set_error("conv_tc: res_mode set but res is NULL"); return CWFA_EINVAL; }
+    if ((reinterpret_cast<uintptr_t>(x_c8) & 15) || (reinterpret_cast<uintptr_t>(w_packed) & 15) ||
+        (out_mode != 3 && (reinterpret_cast<uintptr_t>(out) & 15))) {
+        set_error("conv_tc: pointers must be 16-byte aligned");
+        return CWFA_EINVAL;
+    }
+    EncodeTiledFn encode = get_encode();
+    if (!encode) { set_error("conv_tc: cuTensorMapEncodeTiled not available"); return CWFA_ECUDA; }
+
+    p.Cout = Cout;
     p.w_packed = (const uint8_t*)w_packed; p.bias = bias;
     {
         const int nblks_all = (out_mode == 2 ? 4 : 1) * Cout_p / BN;
@@ -1157,7 +1210,6 @@ static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* b
         p.cpl_x = cpl->x; p.cpl_y = cpl->y; p.cpl_t = cpl->t; p.cpl_perm = cpl->perm; p.cpl_ws = cpl->ws;
         p.cpl_ch = cpl->ch; p.cpl_axis = cpl->axis; p.cpl_inverse = cpl->inverse; p.cpl_kk = cpl->kk; p.cpl_tscale = cpl->tscale;
     }
-    const size_t smem = fixed + (size_t)bs * p.b_bytes;
 
     CUtensorMap tmap;
     const cuuint64_t gdim[4] = {(cuuint64_t)W * 8, (cuuint64_t)H, (cuuint64_t)(Cin_p / 8), (cuuint64_t)N};
@@ -1169,55 +1221,29 @@ static int conv_tc_launch(const void* x_c8, const void* w_packed, const float* b
                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) { set_error("conv_tc: cuTensorMapEncodeTiled failed (%d)", (int)cr); return CWFA_ECUDA; }
 
-    const bool wide = out_mode != 3 && MB * BN > 256;      // > 256 TMEM columns: one CTA per SM anyway
-    typedef void (*KernT)(const CUtensorMap, const TcParams);
-    KernT kern;
-    int ki;
-    // lean epilogue variants: C8 output, no residual, activation none / PReLU
-    const int fast = (out_mode == 0 && res_mode == 0) ? (act == CWFA_ACT_NONE ? 1 : (act == CWFA_ACT_PRELU && slope) ? 2 : 0) : 0;
-    if (stats && (fast == 0 || !wide)) {
-        set_error("conv_tc: fused BatchNorm statistics need the lean epilogue of the wide kernel (C8 output, no residual, act none / PReLU, MB * BN > 256)");
-        return CWFA_EINVAL;
-    }
-    if (out_mode == 3) {
-        const int cplmode = (cpl->t ? 2 : 0) + (cpl->inverse ? 1 : 0);       // 0 fwd, 1 inv, 2 fwd+ext, 3 inv+ext
-        static const KernT table[2][4] = {
-            {conv_tc_kernel<false, 1, false, 0>, conv_tc_kernel<false, 2, false, 0>, conv_tc_kernel<false, 3, false, 0>, conv_tc_kernel<false, 4, false, 0>},
-            {conv_tc_kernel<true, 1, false, 0>, conv_tc_kernel<true, 2, false, 0>, conv_tc_kernel<true, 3, false, 0>, conv_tc_kernel<true, 4, false, 0>}};
-        kern = table[is_bf16 ? 1 : 0][cplmode];
-        ki = 12 + (is_bf16 ? 4 : 0) + cplmode;
-    } else {
-        static const KernT table[2][2][3] = {
-            {{conv_tc_kernel<false, 0, false, 0>, conv_tc_kernel<false, 0, false, 1>, conv_tc_kernel<false, 0, false, 2>},
-             {conv_tc_kernel<false, 0, true, 0>, conv_tc_kernel<false, 0, true, 1>, conv_tc_kernel<false, 0, true, 2>}},
-            {{conv_tc_kernel<true, 0, false, 0>, conv_tc_kernel<true, 0, false, 1>, conv_tc_kernel<true, 0, false, 2>},
-             {conv_tc_kernel<true, 0, true, 0>, conv_tc_kernel<true, 0, true, 1>, conv_tc_kernel<true, 0, true, 2>}}};
-        kern = table[is_bf16 ? 1 : 0][wide ? 1 : 0][fast];
-        ki = (is_bf16 ? 6 : 0) + (wide ? 3 : 0) + fast;
-        if (p.b_resident) {
-            static const KernT table_res[2][3] = {
-                {conv_tc_kernel<false, 0, false, 0, true>, conv_tc_kernel<false, 0, false, 1, true>, conv_tc_kernel<false, 0, false, 2, true>},
-                {conv_tc_kernel<true, 0, false, 0, true>, conv_tc_kernel<true, 0, false, 1, true>, conv_tc_kernel<true, 0, false, 2, true>}};
-            kern = table_res[is_bf16 ? 1 : 0][fast];
-            ki = 20 + (is_bf16 ? 3 : 0) + fast;
-        }
-    }
+    const ConvTcKernel kern = kConvTcKernels[pl.ki];
     static bool attr_done[26] = {};
-    if (!attr_done[ki]) {
+    if (!attr_done[pl.ki]) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        attr_done[ki] = true;
+        attr_done[pl.ki] = true;
     }
-    const int64_t items = (int64_t)p.tiles_x * p.tiles_y * N * ((out_mode == 2 ? 4 : 1) * Cout_p / BN);
-    if (items > 0x7fffffff) { set_error("conv_tc: too many tiles"); return CWFA_EINVAL; }
-    p.total_items = (int)items;
-    // Persistent grid: each CTA walks items blockIdx.x, +grid, ... so TMEM allocation, barrier set-up and the
-    // first-operand TMA latency are paid once per CTA, and (MB*BN <= 128) two accumulator buffers overlap the
-    // MMAs of the next item with this item's epilogue.  The coupling variants keep one item per CTA.
-    p.acc_bufs = (out_mode != 3 && MB * BN <= 128) ? 2 : 1;
-    const int occ = (wide || smem > 113 * 1024) ? 1 : 2;
-    int64_t gx = out_mode == 3 ? items : (items < (int64_t)kNumSMs * occ ? items : (int64_t)kNumSMs * occ);
-    kern<<<(unsigned)gx, wide ? 576 : kThreads, smem, (cudaStream_t)stream>>>(tmap, p);
+    kern<<<(unsigned)pl.grid, pl.wide ? 576 : kThreads, pl.smem, (cudaStream_t)stream>>>(tmap, p);
     return check_launch("conv_tc");
+}
+
+// The plan cwfa_conv_tc / cwfa_conv_tc_bn / cwfa_conv_tc_coupling would launch for these shapes (nothing is launched).
+extern "C" int cwfa_conv_tc_plan(int N, int H, int W, int Cin_p, int Cout_p, int KH, int KW, int BN, int MB, int act, int res_mode,
+                                 int out_mode, int has_slope, int stats, int cpl_inverse, int cpl_ext, int is_bf16, int* plan) {
+    if (!plan) { set_error("conv_tc_plan: plan is NULL"); return CWFA_EINVAL; }
+    TcParams p{};
+    TcPlan pl{};
+    const int cplmode = out_mode == 3 ? (cpl_ext ? 2 : 0) + (cpl_inverse ? 1 : 0) : -1;
+    int rc = conv_tc_plan(p, pl, N, H, W, Cin_p, Cout_p, KH, KW, BN, MB, act, res_mode, out_mode, is_bf16, has_slope != 0, stats != 0,
+                          cplmode);
+    if (rc) return rc;
+    const int v[9] = {pl.ki, p.a_stages, p.b_stages, p.b_resident, p.acc_bufs, pl.wide, (int)pl.grid, p.total_items, (int)pl.smem};
+    for (int i = 0; i < 9; ++i) plan[i] = v[i];
+    return CWFA_OK;
 }
 
 extern "C" int cwfa_conv_tc(const void* x_c8, const void* w_packed, const float* bias, const float* slope,

@@ -175,6 +175,15 @@ class PackedConv:
             self.bias = b
 
 
+def _conv_mb(pc: PackedConv, W: int, mb: Optional[int]) -> int:
+    """M-blocks per tile of ``conv_tc``: ``mb`` if given, else the default for the packed tile width and the image width."""
+    if mb is not None:
+        return mb
+    if pc.BN >= 192 and pc.Cin_p <= 64:
+        return 1          # small-K, wide-N: 128-pixel tiles keep two CTAs per SM (<= 256 TMEM columns each)
+    return 2 if (pc.BN * 2 <= 512 and W > 8) else 1
+
+
 def conv_tc(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[torch.Tensor] = None, res=None, res_mode: int = 0,
             out_nchw: bool = False, mb: Optional[int] = None):
     """Implicit-GEMM convolution on the tensor cores.  Returns a C8 tensor (or NCHW fp32 if out_nchw)."""
@@ -183,10 +192,7 @@ def conv_tc(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[torch.Tensor
     if pc.transposed:
         raise ValueError("use conv_transpose_tc for transposed weights")
     N, H, W = x.N, x.H, x.W
-    if mb is None:
-        mb = 2 if (pc.BN * 2 <= 512 and W > 8) else 1
-        if pc.BN >= 192 and pc.Cin_p <= 64:
-            mb = 1        # small-K, wide-N: 128-pixel tiles keep two CTAs per SM (<= 256 TMEM columns each)
+    mb = _conv_mb(pc, W, mb)
     dev = x.data.device
     if out_nchw:
         out = torch.empty((N, pc.Cout, H, W), device=dev, dtype=torch.float32)
@@ -203,6 +209,24 @@ def conv_tc(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[torch.Tensor
     return out
 
 
+def conv_tc_plan(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[torch.Tensor] = None, res_mode: int = 0,
+                 out_nchw: bool = False, mb: Optional[int] = None, stats: bool = False, coupling=None) -> dict:
+    """The launch plan of ``conv_tc`` (``stats``: of ``conv_tc_bn_stats``' fused-statistics launch) with these arguments, as
+    the library computes it; ``coupling = (inverse, external_shift)`` asks for ``conv_tc_coupling(persistent=False)`` instead.
+    Keys: ki (kernel index 0-25, see include/cwfa_b200.h), a_stages, b_stages, resident, acc_bufs, wide, grid, items, smem."""
+    import ctypes as C
+    if coupling is None:
+        out_mode, bn, mb = (1 if out_nchw else 0), pc.BN, _conv_mb(pc, x.W, mb)
+        inv = ext = 0
+    else:
+        out_mode, bn, mb = 3, pc.Cout_p, (mb if mb is not None else (2 if x.W > 8 else 1))
+        inv, ext = int(bool(coupling[0])), int(bool(coupling[1]))
+    v = (C.c_int * 9)()
+    _lib.call("cwfa_conv_tc_plan", x.N, x.H, x.W, pc.Cin_p, pc.Cout_p, pc.KH, pc.KW, bn, mb, act, res_mode, out_mode,
+              int(slope is not None), int(stats), inv, ext, x.is_bf16, v)
+    return dict(zip(("ki", "a_stages", "b_stages", "resident", "acc_bufs", "wide", "grid", "items", "smem"), list(v)))
+
+
 def conv_tc_bn_stats(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[torch.Tensor] = None, mb: Optional[int] = None):
     """``conv_tc`` (C8 out, no residual, act none / PReLU) that also accumulates the BatchNorm statistics of its activated
     output in the epilogue.  Returns (out, partial, MB) -- feed ``partial`` to ``batchnorm_c8(..., partial=...)`` -- or
@@ -210,10 +234,7 @@ def conv_tc_bn_stats(x: C8, pc: PackedConv, *, act: int = 0, slope: Optional[tor
     if x.Cp != pc.Cin_p or x.kind != pc.kind or pc.transposed:
         raise ValueError("conv_tc_bn_stats: input / weight layout mismatch")
     N, H, W = x.N, x.H, x.W
-    if mb is None:
-        mb = 2 if (pc.BN * 2 <= 512 and W > 8) else 1
-        if pc.BN >= 192 and pc.Cin_p <= 64:
-            mb = 1
+    mb = _conv_mb(pc, W, mb)
     if mb * pc.BN <= 256 or pc.Cout_p != pc.Cout:
         return conv_tc(x, pc, act=act, slope=slope, mb=mb), None, mb
     dev = x.data.device

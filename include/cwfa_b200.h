@@ -160,6 +160,14 @@ int cwfa_conv_tc(const void* x_c8, const void* w_packed, const float* bias, cons
                  const void* res, void* out, int N, int H, int W, int Cin_p, int Cout, int Cout_p,
                  int KH, int KW, int BN, int MB, int act, int res_mode, int out_mode, int is_bf16,
                  void* stream);
+/* The launch plan cwfa_conv_tc (out_mode 0-2), cwfa_conv_tc_bn (stats != 0) or cwfa_conv_tc_coupling (out_mode 3, with the
+ * coupling direction cpl_inverse and shift source cpl_ext) would use for these shapes; has_slope = a PReLU slope pointer is
+ * passed.  Launches nothing.  plan[9] = {kernel index 0-25, A stages, B stages, resident weights, TMEM accumulator buffers,
+ * wide (576-thread) kernel, grid, work items, dynamic shared memory bytes}.  Kernel index: 0-11 ring path
+ * (fp16 | bf16) x (generic | wide) x epilogue (generic, lean none, lean PReLU); 12-19 fused coupling (fp16 | bf16) x
+ * (fwd, inv, fwd + external shift, inv + external shift); 20-25 resident weights (fp16 | bf16) x epilogue. */
+int cwfa_conv_tc_plan(int N, int H, int W, int Cin_p, int Cout_p, int KH, int KW, int BN, int MB, int act, int res_mode,
+                      int out_mode, int has_slope, int stats, int cpl_inverse, int cpl_ext, int is_bf16, int* plan);
 /* cwfa_conv_tc with the BatchNorm statistics of its (activated) output produced by the epilogue -- no separate pass over the
  * tensor (unet.py:100-107: conv -> PReLU -> BatchNorm in batch-statistics mode): one (sum, sum of squares) partial per 32-pixel
  * warp row and channel, plain stores, then a fixed-order two-stage sum (bit-reproducible).  stats_partial:

@@ -6,6 +6,7 @@ import torch.nn.functional as F
 
 from conftest import max_abs, rel_l2
 from oracle.weights import seeded_randn
+from test_gpu_coupling import _coupling_reference
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -187,18 +188,6 @@ def test_conv_tc_skips_zero_weight_blocks():
     assert rel_l2(y[:, 192:], ref[:, 192:]) < 6e-3              # bias only
 
 
-def _coupling_reference(a, x, t_ext, t_scale, ch, inverse, clamp=2.0, k=0.636):
-    s = clamp * k * torch.atan(a[:, :ch])                 # coupling_layers.py:490-500 (a is already divided by nothing: CWFA clamps via atan)
-    t = t_scale * t_ext if t_ext is not None else a[:, ch:2 * ch]
-    if inverse:
-        y = (x - t) * torch.exp(-s)
-        j = -s.sum(dim=(1, 2, 3))
-    else:
-        y = torch.exp(s) * x + t
-        j = s.sum(dim=(1, 2, 3))
-    return y, j
-
-
 @pytest.mark.parametrize("ch,axis,inverse,ext,zero_x", [
     (48, 1, True, False, False), (48, 3, True, False, False), (24, 2, False, False, False), (12, 1, False, True, False),
     (6, 0, True, True, True), (6, 3, False, False, False), (48, 0, True, False, True), (24, 1, True, True, False)])
@@ -221,7 +210,7 @@ def test_fused_coupling_conv_vs_reference(ch, axis, inverse, ext, zero_x, persis
         n_ax = {1: ch, 2: H, 3: W}[axis]
         perm = torch.from_numpy(__import__("numpy").random.RandomState(7).permutation(n_ax)).long()
         xin = xin.index_select(axis, perm)                 # the permutation preceding the coupling (fixed_transforms.py:37-41)
-    y_ref, j_ref = _coupling_reference(a, xin, t_ext, -0.5 ** 0.5 if ext else 1.0, ch, inverse)
+    y_ref, j_ref, _ = _coupling_reference(a, xin, t_ext, -0.5 ** 0.5 if ext else 1.0, ch, inverse)
     pc = tc.PackedConv(w.to(DEV), bias.to(DEV), kind, bn=tc.pad16(cout))
     # "ticket": the persistent kernel reduces its own partial sums (last-CTA finalize); the int32 must come back as zero
     ticket = torch.zeros(1, device=DEV, dtype=torch.int32) if persistent == "ticket" else None
