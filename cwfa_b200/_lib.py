@@ -37,6 +37,7 @@ _SIGS = {
     "cwfa_gate_add_f32": [vp, vp, vp, i64, vp],
     "cwfa_cast_f32_f16": [vp, vp, i64, vp],
     "cwfa_extract_views": [vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, i32, vp],
+    "cwfa_extract_views_c8": [vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, f32, f32, i32, i32, vp],
     "cwfa_attention_gate_f32": [vp, vp, vp, vp, vp, vp, vp, i32, i32, i64, vp],
     "cwfa_tc_kc": [i32],
     "cwfa_tc_pack_weights": [vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp],

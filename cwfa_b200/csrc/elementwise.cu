@@ -723,9 +723,10 @@ __global__ void __launch_bounds__(256) extract_views_kernel(const TIn* __restric
         }
     }
 }
-extern "C" int cwfa_extract_views(const void* image, int image_is_half, const int32_t* coords, float* out, int B, int Hi,
+extern "C" int cwfa_extract_views(const void* image, int image_dtype, const int32_t* coords, float* out, int B, int Hi,
                                   int Wi, int L, int SH, int SW, float mean, float stdv, int normalise, void* stream) {
-    if (B <= 0 || Hi <= 0 || Wi <= 0 || L <= 0 || SH <= 0 || SW <= 0 || (normalise && stdv == 0.f) || (int64_t)B * L > 65535) {
+    if (B <= 0 || Hi <= 0 || Wi <= 0 || L <= 0 || SH <= 0 || SW <= 0 || (normalise && stdv == 0.f) || (int64_t)B * L > 65535 ||
+        image_dtype < 0 || image_dtype > 2) {
         set_error("extract_views: bad arguments");
         return CWFA_EINVAL;
     }
@@ -736,7 +737,9 @@ extern "C" int cwfa_extract_views(const void* image, int image_is_half, const in
     const int threads = work >= 256 ? 256 : (work >= 128 ? 128 : 64);
     if ((SW & 3) == 0 && (reinterpret_cast<uintptr_t>(out) & 15)) { set_error("extract_views: out must be 16-byte aligned"); return CWFA_EINVAL; }
     dim3 grid(gx, B * L);
-    if (image_is_half)
+    if (image_dtype == 2)
+        extract_views_kernel<uint16_t><<<grid, threads, 0, (cudaStream_t)stream>>>((const uint16_t*)image, coords, out, Hi, Wi, L, SH, SW, mean, stdv, normalise);
+    else if (image_dtype == 1)
         extract_views_kernel<__half><<<grid, threads, 0, (cudaStream_t)stream>>>((const __half*)image, coords, out, Hi, Wi, L, SH, SW, mean, stdv, normalise);
     else
         extract_views_kernel<float><<<grid, threads, 0, (cudaStream_t)stream>>>((const float*)image, coords, out, Hi, Wi, L, SH, SW, mean, stdv, normalise);

@@ -14,30 +14,107 @@ from typing import Dict, Optional, Sequence, Tuple
 
 import torch
 
-from . import _lib
+from . import _lib, tc
 from .ops import _stream
+
+
+_IMAGE_DTYPES = {torch.float32: 0, torch.float16: 1, torch.uint16: 2}     # image_dtype codes of cwfa_extract_views(_c8)
 
 
 def extract_views(image: torch.Tensor, lenslet_coords, subimage_shape: Sequence[int], mean: Optional[float] = None,
                   std: Optional[float] = None, debug: bool = False) -> torch.Tensor:
     """``(B,1,Hi,Wi)`` sensor image -> ``(B, n_lenslets, S0, S1)`` stacked views (XLFMDataset.py:212-242) in ONE gather
-    kernel; with ``mean``/``std`` also ``(x - mean) / std`` (CWFA.py:797).  Output is fp32."""
+    kernel; with ``mean``/``std`` also ``(x - mean) / std`` (CWFA.py:797).  Output is fp32.  fp32, fp16 and uint16 (raw
+    sensor) images are read as they are; any other dtype is converted to fp32 first.  For a stream of frames with fixed
+    coordinates see ``LensletLayout``, which uploads them once."""
     if not image.is_cuda:
         raise RuntimeError("cwfa_b200.extract_views needs a CUDA tensor (no CPU fallback)")
     if image.dim() != 4 or image.shape[1] < 1:
         raise ValueError("image must be (B, C>=1, H, W); channel 0 is used, as in the reference")
     img = image[:, 0].contiguous()
-    if img.dtype not in (torch.float32, torch.float16):
+    if img.dtype not in _IMAGE_DTYPES:
         img = img.float()
     coords = torch.as_tensor(lenslet_coords, dtype=torch.int32).reshape(-1, 2).to(image.device).contiguous()
+    norm = mean is not None and std is not None
+    return _views_f32(img, coords, subimage_shape, float(mean) if norm else 0.0, float(std) if norm else 1.0, norm)
+
+
+def _views_f32(img: torch.Tensor, coords: torch.Tensor, subimage_shape, mean: float, std: float, norm: bool) -> torch.Tensor:
     B, Hi, Wi = img.shape
     L = coords.shape[0]
     S0, S1 = int(subimage_shape[0]), int(subimage_shape[1])
-    out = torch.empty((B, L, S0, S1), device=image.device, dtype=torch.float32)
-    norm = mean is not None and std is not None
-    _lib.call("cwfa_extract_views", img.data_ptr(), int(img.dtype == torch.float16), coords.data_ptr(), out.data_ptr(), B, Hi, Wi, L,
-              S0, S1, float(mean) if norm else 0.0, float(std) if norm else 1.0, int(norm), _stream())
+    out = torch.empty((B, L, S0, S1), device=img.device, dtype=torch.float32)
+    _lib.call("cwfa_extract_views", img.data_ptr(), _IMAGE_DTYPES[img.dtype], coords.data_ptr(), out.data_ptr(), B, Hi, Wi, L,
+              S0, S1, mean, std, int(norm), _stream())
     return out
+
+
+class LensletLayout:
+    """The lenslet geometry of a dataset, held once on the device, so that raw sensor frames become views inside a captured
+    CUDA graph or a stream: ``layout = LensletLayout(coords, (512, 512), mean, std)``, then per frame
+    ``layout.views(frame)`` (fp32 NCHW, identical to ``extract_views``) or ``layout.views_c8(frame, kind)`` (the tensor-core
+    engine's input, bitwise equal to ``tc.to_c8(layout.views(frame), kind)`` in one pass without the fp32 views).
+
+    Frames are ``(B, 1, Hi, Wi)`` (channel 0 is used, as in ``extract_views``) or ``(B, Hi, Wi)`` in uint16, float16 or float32,
+    on the layout's device.  Neither method touches the host: no host allocation, no host-to-device copy."""
+
+    def __init__(self, lenslet_coords, subimage_shape: Sequence[int], mean: Optional[float] = None, std: Optional[float] = None,
+                 device="cuda"):
+        coords = torch.as_tensor(lenslet_coords).detach()
+        if coords.dim() != 2 or coords.shape[1] != 2 or coords.shape[0] < 1:
+            raise ValueError(f"lenslet_coords must be (L, 2) (row, col) centres with L >= 1, got shape {tuple(coords.shape)}")
+        if coords.is_floating_point() and not torch.equal(coords, coords.round()):
+            raise ValueError("lenslet_coords must be integer pixel positions")
+        if int(coords.min()) < -2 ** 31 or int(coords.max()) >= 2 ** 31:
+            raise ValueError("lenslet_coords do not fit int32")
+        if len(subimage_shape) != 2 or int(subimage_shape[0]) <= 0 or int(subimage_shape[1]) <= 0:
+            raise ValueError(f"subimage_shape must be two positive view sides, got {tuple(subimage_shape)}")
+        if (mean is None) != (std is None):
+            raise ValueError("give both mean and std (normalised views) or neither")
+        if std is not None and float(std) == 0.0:
+            raise ValueError("std must be non-zero")
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError("cwfa_b200.LensletLayout needs a CUDA device (no CPU fallback)")
+        if device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        self.device = device
+        self.coords = coords.to(torch.int32).to(device).contiguous()
+        self.n_lenslets = int(coords.shape[0])
+        self.subimage_shape = (int(subimage_shape[0]), int(subimage_shape[1]))
+        self.normalise = mean is not None
+        self.mean = float(mean) if self.normalise else 0.0
+        self.std = float(std) if self.normalise else 1.0
+
+    def _frame(self, image: torch.Tensor) -> torch.Tensor:
+        """The frame as a contiguous (B, Hi, Wi) tensor of a supported dtype on the layout's device (a view when it already is)."""
+        if not image.is_cuda:
+            raise RuntimeError("cwfa_b200.LensletLayout needs the frame on a CUDA device (no CPU fallback)")
+        if image.device != self.device:
+            raise ValueError(f"frame on {image.device}, lenslet layout on {self.device}")
+        if image.dtype not in _IMAGE_DTYPES:
+            raise TypeError(f"frames must be uint16, float16 or float32, got {image.dtype}")
+        if image.dim() == 4 and image.shape[1] >= 1:
+            image = image[:, 0]
+        elif image.dim() != 3:
+            raise ValueError(f"frame must be (B, 1, Hi, Wi) or (B, Hi, Wi), got shape {tuple(image.shape)}")
+        if not image.is_contiguous():
+            image = torch.empty(image.shape, device=image.device, dtype=image.dtype).copy_(image)
+        return image
+
+    def views(self, image: torch.Tensor) -> torch.Tensor:
+        """``(B, L, S0, S1)`` fp32 views of the frame, identical to ``extract_views(image, coords, shape, mean, std)``."""
+        return _views_f32(self._frame(image), self.coords, self.subimage_shape, self.mean, self.std, self.normalise)
+
+    def views_c8(self, image: torch.Tensor, kind: str = "bf16") -> tc.C8:
+        """The views as a ``tc.C8`` tensor (``Cp = pad16(L)``; lenslet slots L..Cp-1 are 0) in one pass over the frame."""
+        img = self._frame(image)
+        B, Hi, Wi = img.shape
+        S0, S1 = self.subimage_shape
+        out = tc.C8.empty(B, self.n_lenslets, S0, S1, img.device, kind)
+        _lib.call("cwfa_extract_views_c8", img.data_ptr(), _IMAGE_DTYPES[img.dtype], self.coords.data_ptr(), out.data.data_ptr(),
+                  B, Hi, Wi, self.n_lenslets, out.Cp, S0, S1, self.mean, self.std, int(self.normalise), out.is_bf16, _stream())
+        return out
 
 
 def denormalize(volume: torch.Tensor, mean_vols, std_vols) -> torch.Tensor:

@@ -20,6 +20,7 @@ import torch
 
 from . import modules as Fm
 from . import networks, ops, tc
+from .data import LensletLayout
 from .pipeline import CWFAModel, lrnn_mean_volume
 
 
@@ -138,6 +139,10 @@ class CWFAEngine:
                 out.append((kind, mod, extra, None, 0))
         return out
 
+    def _views_c8(self, views: torch.Tensor, sensor: Optional[LensletLayout]) -> tc.C8:
+        """The conditions in the C8 layout: from fp32 views, or in one pass from a raw sensor frame."""
+        return tc.to_c8(views, self.kind) if sensor is None else sensor.views_c8(views, self.kind)
+
     def _lf(self, n: int, v8: Optional[tc.C8], low_res: Optional[torch.Tensor]) -> tc.C8:
         """LF condition of level n: conditioning net of the views, or (disable_low_res_input) the volume of the level below."""
         if self.dlr:
@@ -255,7 +260,7 @@ class CWFAEngine:
     @torch.no_grad()
     def reconstruct(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], return_all: bool = False,
                     _side_streams=None, zs: Optional[Sequence[Optional[torch.Tensor]]] = None, n_samples: int = 1,
-                    temperature: Optional[float] = None):
+                    temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None):
         """Inverse reconstruction (CWFA.py:865-924); z = 0 unless ``zs[n]`` gives level n's latent sample(s) or
         ``temperature`` (default ``cfg.INN_z_temperature`` = 0) is non-zero (then z ~ ``sample_z_truncated``).
         ``n_samples`` > 1 (batch 1): the reference's multi-sample path (CWFA.py:903-914) -- the coefficients of a level are
@@ -264,14 +269,18 @@ class CWFAEngine:
 
         The LRNN and the coupling coefficients of every level depend only on the views / mean volumes, not on
         each other, so under CUDA-graph capture they are issued on side streams (``_side_streams``) and become
-        parallel branches of the graph; only the four Haar merges are sequential."""
+        parallel branches of the graph; only the four Haar merges are sequential.
+
+        ``sensor``: ``views`` is then a raw sensor frame (``LensletLayout``: uint16 / fp16 / fp32, (B, 1, Hi, Wi) or (B, Hi, Wi)),
+        cropped and normalised straight into the tensor-core input layout; the result is bitwise that of
+        ``reconstruct(sensor.views(frame), ...)``."""
         from .pipeline import sample_z_truncated
         L1 = self.model.n_levels
         T = self.model.cfg.INN_z_temperature if temperature is None else temperature
         B = views.shape[0]
         if n_samples > 1 and B != 1:
             raise ValueError("n_samples > 1 needs batch size 1 (CWFA.py:904)")
-        v8 = tc.to_c8(views, self.kind)
+        v8 = self._views_c8(views, sensor)
         mv_last = lrnn_mean_volume(mean_vols, L1)            # CWFA.py:882: mean_vols_cache[L-2] unless given explicitly
 
         def z_of(n):
@@ -371,13 +380,15 @@ class CWFAEngine:
 
     @torch.no_grad()
     def forward_nll(self, volume: torch.Tensor, views: torch.Tensor, mean_vols: Sequence[torch.Tensor],
-                    low_res_conditions: Optional[Sequence[torch.Tensor]] = None, _side_streams=None):
-        """Forward pyramid + per-level NLL (CWFA.py:966-978); same outputs as CWFAModel.forward_nll.
+                    low_res_conditions: Optional[Sequence[torch.Tensor]] = None, _side_streams=None,
+                    sensor: Optional[LensletLayout] = None):
+        """Forward pyramid + per-level NLL (CWFA.py:966-978); same outputs as CWFAModel.forward_nll.  ``sensor``: ``views`` is
+        a raw sensor frame (see ``reconstruct``).
 
         The conditioning nets and trunks of the four levels depend on the views only, so under CUDA-graph capture
         (``forward_nll_graphed``) they run as parallel branches next to the Haar pyramid of the volume."""
         L1 = self.model.n_levels
-        v8 = None if self.dlr else tc.to_c8(views, self.kind)
+        v8 = None if self.dlr else self._views_c8(views, sensor)
         # Haar pyramid of the volume first (cheap, sequential): lo_n / hi_n of every level
         los, his = [], []
         x = volume
@@ -423,11 +434,14 @@ class CWFAEngine:
         return res
 
     # ---- CUDA-graph replay of the forward pyramid (BASELINE.json configs[2]) ---------------------------------------------
-    def forward_nll_graphed(self, volume: torch.Tensor, views: torch.Tensor, mean_vols: Sequence[torch.Tensor]):
+    def forward_nll_graphed(self, volume: torch.Tensor, views: torch.Tensor, mean_vols: Sequence[torch.Tensor],
+                            sensor: Optional[LensletLayout] = None):
         """``forward_nll`` as one CUDA-graph replay (static shapes; inputs are copied into static buffers, the returned tensors
         are the graph's static outputs, overwritten by the next call): the four levels' conditioning nets / trunks / couplings
-        are parallel branches of the graph."""
-        key = ("nll", tuple(volume.shape), tuple(views.shape), tuple(tuple(m.shape) for m in mean_vols), volume.device.index)
+        are parallel branches of the graph.  ``sensor``: ``views`` is a raw sensor frame; the static input is the frame in its
+        own dtype and the lenslet extraction is part of the graph."""
+        key = ("nll", tuple(volume.shape), tuple(views.shape), tuple(tuple(m.shape) for m in mean_vols), volume.device.index,
+               None if sensor is None else (id(sensor), views.dtype))
         g = self._graphs.get(key)
         if g is None:
             sx, sv, sm = volume.clone(), views.clone(), [m.clone() for m in mean_vols]
@@ -435,14 +449,14 @@ class CWFAEngine:
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 for _ in range(2):
-                    self.forward_nll(sx, sv, sm)
+                    self.forward_nll(sx, sv, sm, sensor=sensor)
             torch.cuda.current_stream().wait_stream(s)
             graph = torch.cuda.CUDAGraph()
             side = [torch.cuda.Stream() for _ in range(self.model.n_levels)] if self.parallel_branches else None
             with torch.cuda.graph(graph):
-                out = self.forward_nll(sx, sv, sm, _side_streams=side)
-            g = self._graphs[key] = (graph, sx, sv, sm, out)
-        graph, sx, sv, sm, out = g
+                out = self.forward_nll(sx, sv, sm, _side_streams=side, sensor=sensor)
+            g = self._graphs[key] = (graph, sx, sv, sm, out, sensor)     # the graph reads the layout's coordinates: keep it alive
+        graph, sx, sv, sm, out = g[:5]
         sx.copy_(volume, non_blocking=True)
         sv.copy_(views, non_blocking=True)
         for d, s_ in zip(sm, mean_vols):
@@ -451,12 +465,14 @@ class CWFAEngine:
         return out
 
     # ---- CUDA-graph replay of the whole frame -------------------------------------------
-    def _graph_slot(self, views: torch.Tensor, mean_vols, slot: int = 0, z_rows: int = 0):
+    def _graph_slot(self, views: torch.Tensor, mean_vols, slot: int = 0, z_rows: int = 0, sensor: Optional[LensletLayout] = None):
         """(graph, static_views, static_mean_vols, static_out, static_zs) for this shape; ``slot`` selects an independent
         instance (own static buffers) so that several frames can be in flight.  ``z_rows`` > 0: the graph takes the latent
         samples of every level as inputs (``z_rows`` rows each; temperature > 0 / multi-sample reconstruction) -- they are
-        sampled outside the graph into the static buffers."""
-        key = (tuple(views.shape), tuple(None if m is None else tuple(m.shape) for m in mean_vols), views.device.index, slot, z_rows)
+        sampled outside the graph into the static buffers.  ``sensor``: the static input is a raw frame in its own dtype and
+        the lenslet extraction is captured in the graph."""
+        key = (tuple(views.shape), tuple(None if m is None else tuple(m.shape) for m in mean_vols), views.device.index, slot, z_rows,
+               None if sensor is None else (id(sensor), views.dtype))
         g = self._graphs.get(key)
         if g is None:
             sv = views.clone()
@@ -470,13 +486,13 @@ class CWFAEngine:
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 for _ in range(2):
-                    self.reconstruct(sv, sm, zs=sz, n_samples=ns)
+                    self.reconstruct(sv, sm, zs=sz, n_samples=ns, sensor=sensor)
             torch.cuda.current_stream().wait_stream(s)
             graph = torch.cuda.CUDAGraph()
             side = [torch.cuda.Stream() for _ in range(self.model.n_levels + 1)] if (self.parallel_branches and not self.dlr) else None
             with torch.cuda.graph(graph):
-                out = self.reconstruct(sv, sm, _side_streams=side, zs=sz, n_samples=ns)
-            g = self._graphs[key] = (graph, sv, sm, out, sz)
+                out = self.reconstruct(sv, sm, _side_streams=side, zs=sz, n_samples=ns, sensor=sensor)
+            g = self._graphs[key] = (graph, sv, sm, out, sz, sensor)      # the graph reads the layout's coordinates: keep it alive
         return g
 
     def _fill_z(self, sz, zs, temperature):
@@ -491,13 +507,14 @@ class CWFAEngine:
 
     def reconstruct_graphed(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]],
                             zs: Optional[Sequence[Optional[torch.Tensor]]] = None, n_samples: int = 1,
-                            temperature: Optional[float] = None) -> torch.Tensor:
+                            temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None) -> torch.Tensor:
         """Same as ``reconstruct`` but replays a captured CUDA graph (static shapes; inputs are copied into
         static buffers, the returned tensor is the graph's static output buffer).  With ``zs`` / a non-zero temperature /
-        ``n_samples`` > 1 the latent samples are graph INPUTS filled before the replay."""
+        ``n_samples`` > 1 the latent samples are graph INPUTS filled before the replay.  ``sensor``: ``views`` is a raw sensor
+        frame, copied as it is into the graph's frame buffer; the lenslet extraction runs inside the graph."""
         T = self.model.cfg.INN_z_temperature if temperature is None else temperature
         z_rows = views.shape[0] * n_samples if (zs is not None or T != 0 or n_samples > 1) else 0
-        graph, sv, sm, out, sz = self._graph_slot(views, mean_vols, z_rows=z_rows)[:5]
+        graph, sv, sm, out, sz = self._graph_slot(views, mean_vols, z_rows=z_rows, sensor=sensor)[:5]
         sv.copy_(views, non_blocking=True)
         for d, s_ in zip(sm, mean_vols):
             if d is not None:
@@ -509,16 +526,20 @@ class CWFAEngine:
 
     # ---- reference-facing call with HOST buffers ------------------------------------------
     def reconstruct_host(self, views_host: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]],
-                         out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
+                         out_host: Optional[torch.Tensor] = None, sensor: Optional[LensletLayout] = None) -> torch.Tensor:
         """views on the HOST (pinned for full speed) -> H2D copy -> graph replay -> D2H copy of the
         reconstructed volume into ``out_host``.  The mean-volume conditions are dataset constants and
-        stay resident on the device.  Returns ``out_host`` (synchronised)."""
+        stay resident on the device.  Returns ``out_host`` (synchronised).  ``sensor``: ``views_host`` is a raw sensor frame,
+        copied in its own dtype (a uint16 frame is a third of the bytes of the fp32 views it becomes)."""
         dev = mean_vols[0].device
-        vd = getattr(self, "_views_dev", None)
-        if vd is None or vd.shape != views_host.shape:
-            vd = self._views_dev = torch.empty(views_host.shape, device=dev, dtype=torch.float32)
+        attr = "_views_dev" if sensor is None else "_frame_dev"
+        dtype = torch.float32 if sensor is None else views_host.dtype
+        vd = getattr(self, attr, None)
+        if vd is None or vd.shape != views_host.shape or vd.dtype != dtype:
+            vd = torch.empty(views_host.shape, device=dev, dtype=dtype)
+            setattr(self, attr, vd)
         vd.copy_(views_host, non_blocking=True)
-        out = self.reconstruct_graphed(vd, mean_vols)
+        out = self.reconstruct_graphed(vd, mean_vols, sensor=sensor)
         if out_host is None:
             out_host = torch.empty(out.shape, dtype=torch.float32, pin_memory=True)
         out_host.copy_(out, non_blocking=True)
@@ -535,16 +556,24 @@ class StreamingReconstructor:
     The mean-volume pyramid is a dataset constant and stays on the device."""
 
     def __init__(self, engine: CWFAEngine, views_shape, mean_vols: Sequence[Optional[torch.Tensor]], depth: int = 2,
-                 out_dtype: torch.dtype = torch.float32):
+                 out_dtype: torch.dtype = torch.float32, sensor: Optional[LensletLayout] = None,
+                 frame_dtype: torch.dtype = torch.uint16):
         """``out_dtype=torch.float16``: host-resident outputs are narrowed on the device (one cast kernel) so the device->host
         transfer carries half the bytes (the reference's own GPU output is fp16 under autocast, CWFA.py:845); the host buffers
-        passed to ``run`` must then be fp16."""
+        passed to ``run`` must then be fp16.
+
+        ``sensor``: the inputs passed to ``run`` are raw sensor frames of shape ``views_shape`` ((B, 1, Hi, Wi) or (B, Hi, Wi))
+        and dtype ``frame_dtype`` (uint16, float16 or float32); they are copied to the device as they are and cropped into
+        views inside each frame's graph.  A uint16 2160 x 2160 frame is 9.3 MB against 30.4 MB of fp32 views."""
         if out_dtype not in (torch.float32, torch.float16):
             raise ValueError("out_dtype must be torch.float32 or torch.float16")
+        if sensor is not None and frame_dtype not in (torch.uint16, torch.float16, torch.float32):
+            raise ValueError("frame_dtype must be torch.uint16, torch.float16 or torch.float32")
         self.eng, self.depth, self.out_dtype = engine, depth, out_dtype
         dev = mean_vols[0].device
-        probe = torch.zeros(views_shape, device=dev, dtype=torch.float32)
-        self.slots = [engine._graph_slot(probe, mean_vols, slot=k)[:4] for k in range(depth)]
+        probe = torch.empty(views_shape, device=dev, dtype=torch.float32 if sensor is None else frame_dtype)
+        (probe.view(torch.int16) if probe.dtype == torch.uint16 else probe).zero_()      # (few torch ops take uint16)
+        self.slots = [engine._graph_slot(probe, mean_vols, slot=k, sensor=sensor)[:4] for k in range(depth)]
         for (graph, sv, sm, out) in self.slots:
             for d, s_ in zip(sm, mean_vols):
                 if d is not None:

@@ -127,10 +127,16 @@ int cwfa_layernorm_chw_f32(const float* x, const float* gamma, const float* beta
 int cwfa_attention_gate_f32(float* x, const float* m, const float* v, const float* w1, const float* b1,
                             const float* w2, const float* b2, int B, int C, int64_t L, void* stream);
 /* Lenslet crop + normalisation in one gather (XLFMDataset.extract_views XLFMDataset.py:212-242 followed by
- * (x - mean) / std, CWFA.py:797): image (B,1,Hi,Wi) fp32 or fp16 -> out (B,L,SH,SW) fp32; coords int32 (L,2) = (row, col)
- * lenslet centres on the device; patches are bottom/right aligned in the view exactly as the reference does. */
-int cwfa_extract_views(const void* image, int image_is_half, const int32_t* coords, float* out, int B, int Hi,
+ * (x - mean) / std, CWFA.py:797): image (B,1,Hi,Wi) -> out (B,L,SH,SW) fp32; image_dtype 0 = fp32, 1 = fp16, 2 = uint16 (a raw
+ * sensor frame); coords int32 (L,2) = (row, col) lenslet centres on the device; patches are bottom/right aligned in the view
+ * exactly as the reference does. */
+int cwfa_extract_views(const void* image, int image_dtype, const int32_t* coords, float* out, int B, int Hi,
                        int Wi, int L, int SH, int SW, float mean, float stdv, int normalise, void* stream);
+/* The same crop + normalisation written straight into the tensor-core input layout (csrc/sensor.cu): out is the C8 tensor
+ * [B][Cp/8][SH][SW][8] bf16 (out_is_bf16) or fp16, 16-byte aligned, Cp >= L and a multiple of 8.  Bitwise equal to
+ * cwfa_extract_views followed by cwfa_nchw_to_c8; lenslet slots L..Cp-1 are 0.  One pass, no fp32 intermediate. */
+int cwfa_extract_views_c8(const void* image, int image_dtype, const int32_t* coords, void* out, int B, int Hi, int Wi, int L,
+                          int Cp, int SH, int SW, float mean, float stdv, int normalise, int out_is_bf16, void* stream);
 /* x += m * 2 * (g - 0.5)   (networks.py:554) */
 int cwfa_gate_add_f32(float* x, const float* m, const float* g, int64_t n, void* stream);
 /* fp32 -> fp16 narrowing of n elements (x, y 16-byte aligned): optional half-size host transfer of a finished volume (the
