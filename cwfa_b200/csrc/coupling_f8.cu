@@ -36,6 +36,7 @@ constexpr uint32_t kOffW = kOffBias + kBiasBytes;            // weights (9*8*BN*
 constexpr int kMaxAStages = 4;
 constexpr int kThreads = 576, kEpiThreads = 512;
 constexpr int kMaxG = 3;                                     // 8-channel groups per epilogue thread (chp8 <= 48, 2 M-blocks, 4-way split)
+constexpr int kSampleBatch = 4;                              // K-sample epilogue: samples whose x loads are issued together
 
 struct F8Params {
     int N, H, W, tiles_x, tiles_y, num_tiles;
@@ -53,11 +54,14 @@ struct F8Params {
     float* sumsq;
     int* ticket;
     int accumulate;
+    int samples;                 // MS kernels: latent samples per condition image (x / y row n * samples + k)
 };
 
 __device__ __forceinline__ float4 ldg128(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 
-template <bool BF16, bool INV, bool EXT>
+// MS: the K-sample inverse variant (engine posterior statistics): one tile's accumulator, i.e. one evaluation of s and t,
+// serves the p.samples latent samples of its condition image.  MS = false is the frame path, unchanged.
+template <bool BF16, bool INV, bool EXT, bool MS = false>
 __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_constant__ CUtensorMap tmap, const F8Params p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -165,6 +169,121 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
             __syncwarp();
             if (++sa == p.a_stages) { sa = 0; pa ^= 1; }
         }
+    } else if constexpr (MS) {
+        // ====================== K-sample epilogue (inverse): 16 warps, same lane / group map as below ======================
+        // s, t (or the external shift) of each of the thread's groups are read once per tile; atan / ex2 run once; then every sample
+        // k of the condition image gets y = (x_k - t) * e with the single-sample kernel's instruction sequence per element, so
+        // sample k is bitwise what a single-sample launch on x_k gives.  One group at a time, x and the external shift loaded after
+        // the accumulator wait: e, t of all three groups plus a sample batch's x do not fit 576 threads' registers unspilled.
+        static_assert(INV, "the K-sample coupling is inverse-only");
+        const int q = warp & 3;
+        const int sub = (warp - 2) >> 2;
+        const int m = q * 32 + lane;
+        const int gpc = p.chp8 >> 3;
+        const int ngroups = 2 * gpc;
+        const uint32_t sstride = (uint32_t)gpc * plane * 8u;         // floats per sample (the launcher checks samples * sstride < 2^31)
+        for (int i = 0; i < my_tiles; ++i) {
+            const int b = i & 1, ph = (i >> 1) & 1;
+            const int t = blockIdx.x + i * gridDim.x;
+            const int n = t / tiles_per_img, rr = t % tiles_per_img;
+            const int h0 = (rr / p.tiles_x) * kTH, w0 = (rr % p.tiles_x) * kTW;
+            const int orow = h0 + (m >> 3);
+            const bool row_ok = orow < p.H;
+            const size_t ibase = (size_t)n * sstride;                   // condition image n (external shift)
+            const size_t xbase = (size_t)n * p.samples * sstride;       // its sample 0
+            uint32_t ooff[kMaxG], soff[kMaxG];
+            bool okg[kMaxG];
+#pragma unroll
+            for (int k = 0; k < kMaxG; ++k) {
+                const int g = sub + 4 * k;
+                const int mb = g >= gpc ? 1 : 0, cg = g - (mb ? gpc : 0);
+                const int ocol = w0 + mb * 8 + (m & 7);
+                const bool ok = g < ngroups && row_ok && ocol < p.W;
+                okg[k] = ok;
+                int srow = orow, scol = ocol;
+                if (ok && p.perm && p.axis == 2) srow = __ldg(p.perm + orow);
+                if (ok && p.perm && p.axis == 3) scol = __ldg(p.perm + ocol);
+                const uint32_t gbase = (uint32_t)cg * plane;
+                ooff[k] = (gbase + (uint32_t)orow * (uint32_t)p.W + (uint32_t)ocol) * 8u;
+                soff[k] = (gbase + (uint32_t)srow * (uint32_t)p.W + (uint32_t)scol) * 8u;
+            }
+            mbar_wait(acc_full(b), ph);
+            tc_fence_after();
+            float sum_a = 0.f;
+#pragma unroll
+            for (int k = 0; k < kMaxG; ++k) {
+                const int g = sub + 4 * k;
+                if (g < ngroups) {                          // warp-uniform
+                    const int mb = g >= gpc ? 1 : 0, cg = g - (mb ? gpc : 0);
+                    uint32_t rs[8], rt[8];
+                    __syncwarp();
+                    const uint32_t ta = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * 256 + mb * p.BN + (cg << 3));
+                    tmem_ld8_nowait(ta, rs);
+                    if constexpr (!EXT) tmem_ld8_nowait(ta + p.chp8, rt);
+                    tmem_ld_wait();
+                    float av[8], ev[8], tv[8];              // EXT: tv = the raw external shift (scaled in the fma below)
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) av[j] = atan_fast(__uint_as_float(rs[j]));
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(ev[j]) : "f"(p.c2 * av[j]));
+                        if constexpr (!EXT) tv[j] = __uint_as_float(rt[j]);
+                    }
+                    if constexpr (EXT) {
+                        const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+                        const float4 t0 = okg[k] ? ldg128(p.t_ext + ibase + ooff[k]) : z4;
+                        const float4 t1 = okg[k] ? ldg128(p.t_ext + ibase + ooff[k] + 4) : z4;
+                        tv[0] = t0.x; tv[1] = t0.y; tv[2] = t0.z; tv[3] = t0.w;
+                        tv[4] = t1.x; tv[5] = t1.y; tv[6] = t1.z; tv[7] = t1.w;
+                    }
+                    float ga = 0.f;
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) ga += av[j];
+                    if (okg[k]) {
+                        sum_a += ga;
+                        // the samples in batches of kSampleBatch: their x loads are in flight together
+#pragma unroll 1
+                        for (int s0 = 0; s0 < p.samples; s0 += kSampleBatch) {
+                            float4 xv[kSampleBatch][2];
+#pragma unroll
+                            for (int u = 0; u < kSampleBatch; ++u) {
+                                if (s0 + u < p.samples) {
+                                    const float* xp = p.x + xbase + (size_t)(s0 + u) * sstride + soff[k];
+                                    xv[u][0] = ldg128(xp);
+                                    xv[u][1] = ldg128(xp + 4);
+                                }
+                            }
+#pragma unroll
+                            for (int u = 0; u < kSampleBatch; ++u) {
+                                if (s0 + u < p.samples) {
+                                    const float xs[8] = {xv[u][0].x, xv[u][0].y, xv[u][0].z, xv[u][0].w,
+                                                         xv[u][1].x, xv[u][1].y, xv[u][1].z, xv[u][1].w};
+                                    float yv[8];
+#pragma unroll
+                                    for (int j = 0; j < 8; ++j) {
+                                        // as the single-sample kernel: (x - tscale * t_ext) is one FFMA there, (x - t) one FADD
+                                        const float d = EXT ? __fmaf_rn(-p.tscale, tv[j], xs[j]) : xs[j] - tv[j];
+                                        yv[j] = d * ev[j];
+                                    }
+                                    float* yp = p.y + xbase + (size_t)(s0 + u) * sstride + ooff[k];
+                                    *reinterpret_cast<float4*>(yp) = make_float4(yv[0], yv[1], yv[2], yv[3]);
+                                    *reinterpret_cast<float4*>(yp + 4) = make_float4(yv[4], yv[5], yv[6], yv[7]);
+                                }
+                            }
+                        }
+                    }
+                }
+            }
+            tc_fence_before();
+            mbar_arrive(acc_empty(b));
+            sum_a = warp_sum(sum_a);
+            if (lane == 0) {
+                float* w = p.ws + ((size_t)t * 16 + (warp - 2)) * 2;
+                w[0] = p.kk * sum_a;
+                w[1] = 0.f;                          // no sum of squares: the inverse direction does not use it
+            }
+        }
+        if (p.ticket) __threadfence();
     } else {
         // ============================ epilogue: 16 warps ============================
         const int q = warp & 3;
@@ -392,6 +511,113 @@ __global__ void __launch_bounds__(256) haar1d_f8_kernel(const float* __restrict_
     }
 }
 
+// ------------------------------------------------------------------------------------------ posterior statistics
+// Split^-1 + IDWT of K latent samples fused with their per-voxel mean and unbiased standard deviation: the K merged volumes
+// exist only in registers.  Sample k: lo row k (or row 0 for every k: lo_shared) and hi row k, hi in F8 (HI_F8) or NCHW.
+// One thread = VEC pixels x 4 channels of lo / hi (= 8 output channels); the two lanes of a pair hold the two halves of one
+// F8 group, so a warp's 128-bit F8 loads cover whole 32-byte pixel groups and its NCHW accesses are 256-byte runs.
+// Welford's update (mean, M2) per output: stable when the spread is many orders below the mean, and M2 stays exactly 0 when
+// every sample gives the same value.  The merged values are the haar1d kernels' (l +- h) * INV_SQRT2, bit for bit.
+template <bool HI_F8, int VEC>
+__global__ void __launch_bounds__(256) haar1d_inv_stats_kernel(const float* __restrict__ lo, const float* __restrict__ hi,
+                                                               float* __restrict__ mean, float* __restrict__ stdev, int K,
+                                                               int lo_shared, int h, int64_t P) {
+    const int G = (h + 7) >> 3;
+    const int64_t Pv = P / VEC;
+    const int64_t total = (int64_t)2 * G * Pv;
+    const int64_t lo_row = lo_shared ? 0 : (int64_t)h * P;
+    const int64_t hi_row = HI_F8 ? (int64_t)G * P * 8 : (int64_t)h * P;
+    const float inv_km1 = 1.f / (float)(K - 1);
+    for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
+        const int half = (int)(idx & 1);
+        const int64_t r = idx >> 1;
+        const int64_t pix = (r % Pv) * VEC;
+        const int g = (int)(r / Pv);
+        const int c0 = g * 8 + half * 4;                   // first lo / hi channel of this thread
+        float mu[4][2][VEC], m2[4][2][VEC];                // [channel][even / odd output][pixel]
+        float lv[4][VEC];
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+#pragma unroll
+            for (int v = 0; v < VEC; ++v) { mu[j][0][v] = mu[j][1][v] = m2[j][0][v] = m2[j][1][v] = 0.f; lv[j][v] = 0.f; }
+#pragma unroll 1
+        for (int k = 0; k < K; ++k) {
+            if (k == 0 || !lo_shared) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (c0 + j < h) {
+                        const float* lp = lo + (int64_t)k * lo_row + (int64_t)(c0 + j) * P + pix;
+                        if constexpr (VEC == 4) {
+                            const float4 l4 = __ldg(reinterpret_cast<const float4*>(lp));
+                            lv[j][0] = l4.x; lv[j][1] = l4.y; lv[j][2] = l4.z; lv[j][3] = l4.w;
+                        } else {
+                            lv[j][0] = __ldg(lp);
+                        }
+                    }
+                }
+            }
+            float hv[4][VEC];
+            if constexpr (HI_F8) {
+#pragma unroll
+                for (int v = 0; v < VEC; ++v) {
+                    const float4 h4 = __ldg(reinterpret_cast<const float4*>(hi + (int64_t)k * hi_row + (((int64_t)g * P + pix + v) * 8) + half * 4));
+                    hv[0][v] = h4.x; hv[1][v] = h4.y; hv[2][v] = h4.z; hv[3][v] = h4.w;
+                }
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (c0 + j < h) {
+                        const float* hp = hi + (int64_t)k * hi_row + (int64_t)(c0 + j) * P + pix;
+                        if constexpr (VEC == 4) {
+                            const float4 h4 = __ldg(reinterpret_cast<const float4*>(hp));
+                            hv[j][0] = h4.x; hv[j][1] = h4.y; hv[j][2] = h4.z; hv[j][3] = h4.w;
+                        } else {
+                            hv[j][0] = __ldg(hp);
+                        }
+                    } else {
+#pragma unroll
+                        for (int v = 0; v < VEC; ++v) hv[j][v] = 0.f;
+                    }
+                }
+            }
+            const float rk = 1.f / (float)(k + 1);
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+#pragma unroll
+                for (int v = 0; v < VEC; ++v) {
+                    // __fmul_rn: the merged value is rounded once, as the merge kernels store it; a product contracted into
+                    // the subtractions below would leave its rounding residual in M2 (std != 0 for identical samples)
+                    const float x2[2] = {__fmul_rn(lv[j][v] + hv[j][v], INV_SQRT2), __fmul_rn(lv[j][v] - hv[j][v], INV_SQRT2)};
+#pragma unroll
+                    for (int e = 0; e < 2; ++e) {
+                        const float d = x2[e] - mu[j][e][v];
+                        mu[j][e][v] = fmaf(d, rk, mu[j][e][v]);
+                        m2[j][e][v] = fmaf(d, x2[e] - mu[j][e][v], m2[j][e][v]);
+                    }
+                }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (c0 + j < h) {
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    const int64_t o = (int64_t)(2 * (c0 + j) + e) * P + pix;
+                    float sd[VEC];
+#pragma unroll
+                    for (int v = 0; v < VEC; ++v) sd[v] = sqrtf(fmaxf(m2[j][e][v], 0.f) * inv_km1);
+                    if constexpr (VEC == 4) {
+                        *reinterpret_cast<float4*>(mean + o) = make_float4(mu[j][e][0], mu[j][e][1], mu[j][e][2], mu[j][e][3]);
+                        *reinterpret_cast<float4*>(stdev + o) = make_float4(sd[0], sd[1], sd[2], sd[3]);
+                    } else {
+                        mean[o] = mu[j][e][0];
+                        stdev[o] = sd[0];
+                    }
+                }
+            }
+        }
+    }
+}
+
 // NCHW <-> F8 with an optional channel map: F8 slot j holds NCHW channel map[j] (to_f8) / NCHW channel c reads F8 slot map[c]
 // (to_nchw).  map == NULL: identity.  4 pixels per thread (128-bit NCHW accesses).
 template <bool TO_F8>
@@ -466,6 +692,25 @@ extern "C" int cwfa_haar1d_inv_f8(const float* lo, const float* hi_f8, float* x,
     haar1d_f8_kernel<true><<<grid_for((int64_t)B * ((h + 7) / 8) * (P / 4)), 256, 0, (cudaStream_t)stream>>>(lo, hi_f8, x, nullptr, B, h, P);
     return check_launch("haar1d_inv_f8");
 }
+// Posterior statistics of the last merge: see haar1d_inv_stats_kernel.  lo: K rows (lo_shared = 0) or one row for all samples;
+// hi: K rows, F8 (hi_f8 = 1) or NCHW; mean / std: one (C, P) volume each.  F8 needs P % 4 == 0 and 16-byte aligned pointers;
+// NCHW uses 128-bit accesses when P % 4 == 0 and they are aligned, scalar ones otherwise.
+extern "C" int cwfa_haar1d_inv_stats(const float* lo, int lo_shared, const float* hi, int hi_f8, float* mean, float* stdev, int K, int C,
+                                     int64_t P, void* stream) {
+    const bool vec = (P & 3) == 0 && aligned16(lo) && aligned16(hi) && aligned16(mean) && aligned16(stdev);
+    if (K < 2 || C <= 0 || (C & 1) || P <= 0 || !lo || !hi || !mean || !stdev || (hi_f8 && !vec)) {
+        set_error("haar1d_inv_stats: needs K >= 2 samples, even C, and for an F8 detail half P %% 4 == 0 and 16-byte aligned pointers");
+        return CWFA_EINVAL;
+    }
+    const int h = C / 2;
+    const int64_t work = (int64_t)2 * ((h + 7) / 8) * (vec ? P / 4 : P);
+    const int grid = grid_for(work);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (hi_f8) haar1d_inv_stats_kernel<true, 4><<<grid, 256, 0, st>>>(lo, hi, mean, stdev, K, lo_shared, h, P);
+    else if (vec) haar1d_inv_stats_kernel<false, 4><<<grid, 256, 0, st>>>(lo, hi, mean, stdev, K, lo_shared, h, P);
+    else haar1d_inv_stats_kernel<false, 1><<<grid, 256, 0, st>>>(lo, hi, mean, stdev, K, lo_shared, h, P);
+    return check_launch("haar1d_inv_stats");
+}
 extern "C" int cwfa_nchw_to_f8(const float* x, const int32_t* map, float* y_f8, int B, int C, int64_t P, void* stream) {
     if (B <= 0 || C <= 0 || P <= 0 || (P & 3) || !aligned16(x) || !aligned16(y_f8)) { set_error("nchw_to_f8: bad arguments (P %% 4 == 0, aligned pointers)"); return CWFA_EINVAL; }
     f8_convert_kernel<true><<<grid_for((int64_t)B * ((C + 7) / 8) * (P / 4)), 256, 0, (cudaStream_t)stream>>>(x, y_f8, map, B, C, P);
@@ -477,32 +722,33 @@ extern "C" int cwfa_f8_to_nchw(const float* x_f8, const int32_t* map, float* y, 
     return check_launch("f8_to_nchw");
 }
 
-// Last conv of a coupling sub-network + affine coupling on the F8 detail half.  w_packed: cwfa_tc_pack_weights output for a
-// 3x3 conv 64 -> BN channels in ONE n-block whose columns are [s of slot 0..chp8-1 | t of slot 0..chp8-1] (or s alone when
-// ct != NULL), slots = storage channels of the F8 tensors (chp8 = 8 * ceil(ch / 8); padding slots: zero weights and bias).
-// cx: F8 input (NULL = zeros, inverse only); cy: F8 output; ct: F8 external shift or NULL; perm: int32 row (perm_axis 2) or
-// column (perm_axis 3) gather indices applied to cx, or NULL.  workspace / logdet / sumsq / accumulate / ticket as in
-// cwfa_coupling_tc (ticket may be NULL: reduce with cwfa_coupling_finalize over cwfa_coupling_tc_tiles(H, W) partials).
-extern "C" int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
-                                const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
-                                float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
-                                int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream) {
+// Shared launcher of cwfa_coupling_f8 (samples == 1) and cwfa_coupling_f8_samples.
+static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_packed, const float* bias, int N, int samples, int H,
+                              int W, int BN, int chp8, const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm,
+                              int perm_axis, float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq,
+                              int accumulate, int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream) {
+    const bool ms = samples > 1;
+    if (samples < 1 || (ms && (!inverse || !cx || sumsq || (int64_t)samples * chp8 * H * W >= (1ll << 31)))) {
+        set_error("%s: samples must be >= 1; with samples > 1 the coupling is inverse-only, needs x, has no sum of squares, and "
+                  "samples * chp8 * H * W must stay below 2^31", name);
+        return CWFA_EINVAL;
+    }
     if (N <= 0 || H <= 0 || W <= 0 || (int64_t)chp8 * H * W >= (1ll << 31) || !cy || !workspace || chp8 <= 0 || chp8 > 48 || (chp8 & 7) ||
         BN > kMaxBN || (BN % 16) || (ct ? BN < chp8 : BN < 2 * chp8) || (perm && perm_axis != 2 && perm_axis != 3) || (!cx && !inverse) ||
         (ticket && !logdet) || in_chunk_off < 0 || in_chunk_off + kChunks > in_total_chunks) {
-        set_error("coupling_f8: unsupported arguments (needs 64 -> BN <= 96 in one n-block, chp8 <= 48 multiple of 8, row / column perms only)");
+        set_error("%s: unsupported arguments (needs 64 -> BN <= 96 in one n-block, chp8 <= 48 multiple of 8, row / column perms only)", name);
         return CWFA_EINVAL;
     }
     if ((reinterpret_cast<uintptr_t>(b_c8) & 15) || (reinterpret_cast<uintptr_t>(w_packed) & 15) || !aligned16(cy) || (cx && !aligned16(cx)) ||
         (ct && !aligned16(ct))) {
-        set_error("coupling_f8: pointers must be 16-byte aligned");
+        set_error("%s: pointers must be 16-byte aligned", name);
         return CWFA_EINVAL;
     }
     F8Params p{};
     p.N = N; p.H = H; p.W = W;
     p.tiles_x = ceil_div(W, kTW); p.tiles_y = ceil_div(H, kTH);
     const int64_t nt = (int64_t)p.tiles_x * p.tiles_y * N;
-    if (nt > 0x7fffffff) { set_error("coupling_f8: too many tiles"); return CWFA_EINVAL; }
+    if (nt > 0x7fffffff) { set_error("%s: too many tiles", name); return CWFA_EINVAL; }
     p.num_tiles = (int)nt;
     p.BN = BN; p.chp8 = chp8; p.axis = perm ? perm_axis : 0;
     p.w = (const uint8_t*)w_packed; p.bias = bias; p.x = cx; p.y = cy; p.t_ext = ct; p.perm = perm; p.ws = workspace;
@@ -510,7 +756,7 @@ extern "C" int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const fl
     p.kk = inverse ? -kk : kk;
     p.c2 = (inverse ? -kk : kk) * 1.4426950408889634f;
     p.tscale = t_scale;
-    p.logdet = logdet; p.sumsq = sumsq; p.ticket = ticket; p.accumulate = accumulate;
+    p.logdet = logdet; p.sumsq = sumsq; p.ticket = ticket; p.accumulate = accumulate; p.samples = samples;
     CUtensorMap tmap;
     p.in_chunk_off = in_chunk_off;
     int rc = make_c8_tensor_map(&tmap, b_c8, N, in_total_chunks, H, W, kBW, kBH, kChunks, is_bf16);
@@ -519,10 +765,13 @@ extern "C" int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const fl
     static const KernT table[2][4] = {
         {coupling_f8_kernel<false, false, false>, coupling_f8_kernel<false, true, false>, coupling_f8_kernel<false, false, true>, coupling_f8_kernel<false, true, true>},
         {coupling_f8_kernel<true, false, false>, coupling_f8_kernel<true, true, false>, coupling_f8_kernel<true, false, true>, coupling_f8_kernel<true, true, true>}};
+    static const KernT table_ms[2][2] = {
+        {coupling_f8_kernel<false, true, false, true>, coupling_f8_kernel<false, true, true, true>},
+        {coupling_f8_kernel<true, true, false, true>, coupling_f8_kernel<true, true, true, true>}};
     const int mode = (ct ? 2 : 0) + (inverse ? 1 : 0);
-    KernT kern = table[is_bf16 ? 1 : 0][mode];
-    static bool attr_done[8] = {false, false, false, false, false, false, false, false};
-    const int ki = (is_bf16 ? 4 : 0) + mode;
+    KernT kern = ms ? table_ms[is_bf16 ? 1 : 0][ct ? 1 : 0] : table[is_bf16 ? 1 : 0][mode];
+    static bool attr_done[12] = {false, false, false, false, false, false, false, false, false, false, false, false};
+    const int ki = ms ? 8 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : (is_bf16 ? 4 : 0) + mode;
     if (!attr_done[ki]) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         attr_done[ki] = true;
@@ -534,5 +783,33 @@ extern "C" int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const fl
     const size_t smem_bytes = 1024 + p.off_a + (size_t)p.a_stages * kA1Bytes;
     const int grid = p.num_tiles < kNumSMs ? p.num_tiles : kNumSMs;
     kern<<<grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(tmap, p);
-    return check_launch("coupling_f8");
+    return check_launch(name);
+}
+
+// ---- C ABI: the coupling kernels --------------------------------------------------------------------------------------
+// Last conv of a coupling sub-network + affine coupling on the F8 detail half.  w_packed: cwfa_tc_pack_weights output for a
+// 3x3 conv 64 -> BN channels in ONE n-block whose columns are [s of slot 0..chp8-1 | t of slot 0..chp8-1] (or s alone when
+// ct != NULL), slots = storage channels of the F8 tensors (chp8 = 8 * ceil(ch / 8); padding slots: zero weights and bias).
+// cx: F8 input (NULL = zeros, inverse only); cy: F8 output; ct: F8 external shift or NULL; perm: int32 row (perm_axis 2) or
+// column (perm_axis 3) gather indices applied to cx, or NULL.  workspace / logdet / sumsq / accumulate / ticket as in
+// cwfa_coupling_tc (ticket may be NULL: reduce with cwfa_coupling_finalize over cwfa_coupling_tc_tiles(H, W) partials).
+extern "C" int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
+                                const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                                float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
+                                int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream) {
+    return coupling_f8_launch("coupling_f8", b_c8, w_packed, bias, N, 1, H, W, BN, chp8, cx, cy, ct, t_scale, perm, perm_axis, clamp,
+                              k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks, in_chunk_off, is_bf16, stream);
+}
+// cwfa_coupling_f8 with ``samples`` latent samples per condition image (inverse only): cx / cy hold N * samples F8 rows, row
+// n * samples + k being sample k of condition image n; b_c8, ct and the log-det stay per condition image (N rows).  s and t
+// are computed once per tile and applied to every sample; sample k's output is bitwise that of cwfa_coupling_f8 on its row.
+// sumsq must be NULL.  samples == 1 is cwfa_coupling_f8.
+extern "C" int cwfa_coupling_f8_samples(const void* b_c8, const void* w_packed, const float* bias, int N, int samples, int H, int W,
+                                        int BN, int chp8, const float* cx, float* cy, const float* ct, float t_scale,
+                                        const int32_t* perm, int perm_axis, float clamp, float k_atan, int inverse, float* workspace,
+                                        float* logdet, float* sumsq, int accumulate, int32_t* ticket, int in_total_chunks,
+                                        int in_chunk_off, int is_bf16, void* stream) {
+    return coupling_f8_launch("coupling_f8_samples", b_c8, w_packed, bias, N, samples, H, W, BN, chp8, cx, cy, ct, t_scale, perm,
+                              perm_axis, clamp, k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks,
+                              in_chunk_off, is_bf16, stream);
 }

@@ -309,22 +309,7 @@ class CWFAEngine:
             return (outs, jacs) if return_all else vol
         jobs = [lambda: self.lrnn(v8, mv_last)] + [(lambda n=n: self._level_detail_inverse(n, self._lf(n, v8, None), mean_vols[n], z_of(n), B))
                                                     for n in range(L1 - 1, -1, -1)]
-        if _side_streams:
-            main = torch.cuda.current_stream()
-            fork = torch.cuda.Event()
-            fork.record(main)
-            results, joins = [], []
-            for st, job in zip(_side_streams, jobs):
-                st.wait_event(fork)
-                with torch.cuda.stream(st):
-                    results.append(job())
-                    ev = torch.cuda.Event()
-                    ev.record(st)
-                joins.append(ev)
-            for ev in joins:
-                main.wait_event(ev)
-        else:
-            results = [job() for job in jobs]
+        results = self._run_jobs(jobs, _side_streams)
         vol = results[0]
         outs, jacs = {L1: vol}, {}
         for k, n in enumerate(range(L1 - 1, -1, -1)):
@@ -332,6 +317,152 @@ class CWFAEngine:
             vol = merge(vol, hi)                     # Split^-1 + IDWT: the only sequential part of the pyramid
             outs[n], jacs[n] = vol, jac
         return (outs, jacs) if return_all else vol
+
+    @staticmethod
+    def _run_jobs(jobs, side_streams):
+        """Runs independent jobs in order, or each on its own side stream (forked from and joined back into the current
+        stream: parallel branches under CUDA-graph capture).  Returns their results in order."""
+        if not side_streams:
+            return [job() for job in jobs]
+        main = torch.cuda.current_stream()
+        fork = torch.cuda.Event()
+        fork.record(main)
+        results, joins = [], []
+        for st, job in zip(side_streams, jobs):
+            st.wait_event(fork)
+            with torch.cuda.stream(st):
+                results.append(job())
+                ev = torch.cuda.Event()
+                ev.record(st)
+            joins.append(ev)
+        for ev in joins:
+            main.wait_event(ev)
+        return results
+
+    # ---- posterior statistics: per-voxel mean and standard deviation over K latent samples ------------------------------
+    def _level_detail_samples(self, n, lf8, mean_vol, z):
+        """Detail halves of level n for the K latent samples ``z`` (K rows) of one frame: ("f8", K-row F8 tensor) on the F8 plan
+        (batched trunks, one K-sample coupling per block: s and t computed once), else the K-row NCHW path of
+        ``_level_detail_inverse``.  Sample k is what ``_level_detail_inverse`` gives for ``z[k:k+1]`` (bitwise on the F8 plan)."""
+        K = z.shape[0]
+        plan = self.levels[n]["f8"] if (self.use_f8 and (lf8.H * lf8.W) % 4 == 0) else None
+        if plan is None:
+            return self._level_detail_inverse(n, lf8, mean_vol, z, K)[0]
+        items = self._trunks(n, lf8)
+        hi = tc.to_f8(z, plan["storage_from_z"])
+        mv8 = None if mean_vol is None else tc.to_f8(mean_vol)
+        jac, tickets = self._jac_and_tickets(lf8.N, lf8.data.device)          # log-det: computed by the kernels, not returned
+        pending, k = None, 0
+        pcs = plan["out"]
+        ci = len(pcs)
+        for item in reversed(items):
+            if item[0] == "cat":
+                ci -= 1
+                _, mod, sub, b8, off = item
+                first = not sub.normal
+                perm, axis = (None, 0) if pending is None else (ops.perm_i32(pending[0], b8.data.device), pending[1])
+                hi = tc.coupling_f8_samples(b8, pcs[ci], hi, K, ch=mod.channels, clamp=mod.clamp, t_ext8=mv8 if first else None,
+                                            t_scale=(-1.0 / math.sqrt(2)) if first else 1.0, perm=perm, perm_axis=axis,
+                                            logdet=jac, ticket=tickets[k:k + 1], chunk_off=off)
+                pending, k = None, (k + 1) % tickets.numel()
+            elif item[2] != 1:                                  # row / column permutation: gathered by the next coupling
+                pending = (item[1].perm_inv, item[2])
+        if pending is not None:
+            hi = self._permute_f8(hi, plan["ch"], pending[0], pending[1])
+        return ("f8", hi)
+
+    def _posterior_check(self, views, n_samples, zs):
+        if self.dlr:
+            raise ValueError("posterior statistics need independent levels: with disable_low_res_input each level is conditioned "
+                             "on the volume reconstructed below it, so the samples are not a chain of independent levels")
+        if int(n_samples) < 2:
+            raise ValueError("posterior statistics need n_samples >= 2")
+        if views.shape[0] != 1:
+            raise ValueError("posterior statistics take one frame (batch size 1, CWFA.py:904)")
+        if zs is not None:
+            for n, z in enumerate(zs):
+                if z is not None and z.shape[0] != int(n_samples):
+                    raise ValueError(f"zs[{n}] has {z.shape[0]} rows, expected n_samples = {int(n_samples)}")
+
+    @torch.no_grad()
+    def reconstruct_posterior(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], n_samples: int,
+                              temperature: Optional[float] = None, zs: Optional[Sequence[Optional[torch.Tensor]]] = None,
+                              sensor: Optional[LensletLayout] = None, _side_streams=None):
+        """Per-voxel posterior mean and unbiased standard deviation over ``n_samples`` = K >= 2 latent samples of one frame:
+        ``(mean, std)``, each (1, D, H, W) fp32.  Sample k's volume V_k is ``reconstruct(views, mean_vols, zs=[z_n[k:k+1]])``
+        with ``z_n`` = ``zs[n]`` (K rows) or, for levels without one, K draws of ``sample_z_truncated(temperature)``
+        (default ``cfg.INN_z_temperature``; temperature 0: z = 0, so std = 0).  mean = sum_k V_k / K,
+        std = sqrt(sum_k (V_k - mean)^2 / (K - 1)).
+
+        The LRNN, the conditioning nets and the sub-network trunks run once for all samples; every coupling of the F8 levels
+        computes its s and t once and applies them to the K samples; the last merge computes the statistics in registers, so
+        the K full-resolution volumes are never written.  Not for ``disable_low_res_input`` models (their levels are not
+        independent).  ``sensor``: ``views`` is a raw sensor frame (see ``reconstruct``)."""
+        from .pipeline import sample_z_truncated
+        self._posterior_check(views, n_samples, zs)
+        K = int(n_samples)
+        L1 = self.model.n_levels
+        T = self.model.cfg.INN_z_temperature if temperature is None else temperature
+        v8 = self._views_c8(views, sensor)
+        mv_last = lrnn_mean_volume(mean_vols, L1)
+
+        def z_of(n):
+            if zs is not None and zs[n] is not None:
+                return zs[n]
+            shape = (K,) + tuple(self.model.conv_inn[n].global_out_shapes[0])
+            if T != 0:
+                return sample_z_truncated(shape, device=views.device, temperature=T)
+            return torch.zeros(shape, device=views.device, dtype=torch.float32)
+
+        jobs = [lambda: self.lrnn(v8, mv_last)] + [(lambda n=n: self._level_detail_samples(n, self._lf(n, v8, None), mean_vols[n], z_of(n)))
+                                                    for n in range(L1 - 1, -1, -1)]
+        results = self._run_jobs(jobs, _side_streams)
+        vol = results[0]
+        for k, n in enumerate(range(L1 - 1, -1, -1)):
+            hi = results[1 + k]
+            hi = hi[1] if isinstance(hi, tuple) else hi
+            if n == 0:
+                return tc.haar1d_merge_stats(vol, hi)            # one LRNN row is shared when level 0 is the only flow level
+            if vol.shape[0] != K:
+                vol = vol.expand(K, -1, -1, -1).contiguous()
+            vol = tc.haar1d_merge_f8(vol, hi) if hi.dim() == 5 else ops.haar1d_merge(vol, hi)
+
+    def reconstruct_posterior_graphed(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], n_samples: int,
+                                      temperature: Optional[float] = None, zs: Optional[Sequence[Optional[torch.Tensor]]] = None,
+                                      sensor: Optional[LensletLayout] = None):
+        """``reconstruct_posterior`` as one CUDA-graph replay.  The latent samples are graph inputs (K rows per level), filled
+        before each replay from ``zs`` or fresh ``sample_z_truncated`` draws as in ``reconstruct_graphed``; the LRNN and the
+        levels are parallel branches.  The returned (mean, std) are the graph's static outputs, overwritten by the next call."""
+        self._posterior_check(views, n_samples, zs)
+        K = int(n_samples)
+        T = self.model.cfg.INN_z_temperature if temperature is None else temperature
+        key = ("posterior", tuple(views.shape), tuple(None if m is None else tuple(m.shape) for m in mean_vols), views.device.index, K,
+               None if sensor is None else (id(sensor), views.dtype))
+        g = self._graphs.get(key)
+        if g is None:
+            sv = views.clone()
+            sm = [None if m is None else m.clone() for m in mean_vols]
+            sz = [torch.zeros((K,) + tuple(self.model.conv_inn[n].global_out_shapes[0]), device=views.device, dtype=torch.float32)
+                  for n in range(self.model.n_levels)]
+            s = torch.cuda.Stream()
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                for _ in range(2):
+                    self.reconstruct_posterior(sv, sm, K, zs=sz, sensor=sensor)
+            torch.cuda.current_stream().wait_stream(s)
+            graph = torch.cuda.CUDAGraph()
+            side = [torch.cuda.Stream() for _ in range(self.model.n_levels + 1)] if self.parallel_branches else None
+            with torch.cuda.graph(graph):
+                out = self.reconstruct_posterior(sv, sm, K, zs=sz, sensor=sensor, _side_streams=side)
+            g = self._graphs[key] = (graph, sv, sm, out, sz, sensor)    # the graph reads the layout's coordinates: keep it alive
+        graph, sv, sm, out, sz = g[:5]
+        sv.copy_(views, non_blocking=True)
+        for d, s_ in zip(sm, mean_vols):
+            if d is not None:
+                d.copy_(s_, non_blocking=True)
+        self._fill_z(sz, zs, T)
+        graph.replay()
+        return out
 
     def _level_forward_f8(self, n, plan, hi8, lf8, mean_vol):
         ch = plan["ch"]

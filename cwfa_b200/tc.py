@@ -530,6 +530,49 @@ def coupling_f8(b: C8, pc: PackedConv, x8: Optional[torch.Tensor], *, ch: int, i
     return y
 
 
+def coupling_f8_samples(b: C8, pc: PackedConv, x8: torch.Tensor, samples: int, *, ch: int, clamp: float = 2.0, k_atan: float = 0.636,
+                        t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0, perm: Optional[torch.Tensor] = None,
+                        perm_axis: int = 0, logdet: torch.Tensor = None, accumulate: bool = True,
+                        ticket: Optional[torch.Tensor] = None, chunk_off: int = 0) -> torch.Tensor:
+    """Inverse ``coupling_f8`` for ``samples`` latent samples of each of the ``b.N`` condition images: ``x8`` has
+    ``b.N * samples`` F8 rows (row n * samples + k = sample k of image n).  s and t are evaluated once per tile for all samples;
+    sample k's output is bitwise ``coupling_f8`` on row k.  ``t_ext8`` and ``logdet`` are per condition image."""
+    if chunk_off * 8 + 64 > b.Cp or pc.Cin_p != 64 or pc.KH != 3 or pc.KW != 3 or b.kind != pc.kind or pc.BN != pc.Cout_p:
+        raise ValueError("coupling_f8_samples: needs a 3x3 conv from 64 hidden channels packed in one n-block")
+    N, H, W = b.N, b.H, b.W
+    c8 = ch8(ch)
+    if tuple(x8.shape) != (N * samples, c8 // 8, H, W, 8):
+        raise ValueError(f"coupling_f8_samples: x8 has shape {tuple(x8.shape)}, expected {(N * samples, c8 // 8, H, W, 8)}")
+    y = torch.empty_like(x8)
+    tiles = _lib.load().cwfa_coupling_tc_tiles(H, W)
+    ws = torch.empty(2 * N * tiles, device=b.data.device, dtype=torch.float32)
+    _lib.call("cwfa_coupling_f8_samples", b.data.data_ptr(), pc.packed.data_ptr(), _p(pc.bias), N, int(samples), H, W, pc.BN, c8,
+              x8.data_ptr(), y.data_ptr(), _p(t_ext8), float(t_scale), _p(perm), int(perm_axis), float(clamp), float(k_atan), 1,
+              ws.data_ptr(), logdet.data_ptr(), None, int(accumulate), _p(ticket), b.Cp // 8, int(chunk_off), b.is_bf16, _stream())
+    if ticket is None:
+        _lib.call("cwfa_coupling_finalize", ws.data_ptr(), logdet.data_ptr(), None, N, tiles, int(accumulate), _stream())
+    return y
+
+
+def haar1d_merge_stats(lo: torch.Tensor, hi: torch.Tensor):
+    """Split^-1 + IDWT of K >= 2 latent samples with only their statistics written: ``lo`` (K or 1, h, H, W) -- one row is
+    shared by every sample -- and the K-row detail half ``hi`` in F8 (K, ceil(h/8), H, W, 8) or NCHW (K, h, H, W).  Returns
+    the per-voxel mean and unbiased standard deviation of the K merged (1, 2h, H, W) volumes."""
+    lo = _ck(lo, "lo")
+    hi = _ck(hi, "hi")
+    L, h, H, W = lo.shape
+    K = hi.shape[0]
+    f8 = hi.dim() == 5
+    want = (K, ch8(h) // 8, H, W, 8) if f8 else (K, h, H, W)
+    if tuple(hi.shape) != want or L not in (1, K):
+        raise ValueError(f"haar1d_merge_stats: lo {tuple(lo.shape)} and detail half {tuple(hi.shape)} do not match")
+    mean = torch.empty((1, 2 * h, H, W), device=lo.device, dtype=torch.float32)
+    std = torch.empty_like(mean)
+    _lib.call("cwfa_haar1d_inv_stats", lo.data_ptr(), int(L == 1), hi.data_ptr(), int(f8), mean.data_ptr(), std.data_ptr(), K, 2 * h,
+              H * W, _stream())
+    return mean, std
+
+
 def resblock_tc_batched(x: C8, sets, in_chunk_offs=None) -> C8:
     """The fused trunk block (``resblock_tc``) for several INDEPENDENT sub-networks in one launch: ``sets`` = [(p3, p1), ...]
     (<= 5); set k reads the 64-channel slice at chunk ``in_chunk_offs[k]`` (default 8 k) of ``x`` and writes slice k of the

@@ -290,6 +290,19 @@ int cwfa_coupling_f8(const void* b_c8, const void* w_packed, const float* bias, 
                      const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
                      float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
                      int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream);
+/* cwfa_coupling_f8 for `samples` latent samples of each condition image (inverse only; posterior statistics): cx / cy hold
+ * N * samples F8 rows, row n * samples + k = sample k of condition image n; b_c8, ct and logdet stay per condition image.  s and
+ * t are computed once per tile and applied to every sample, each sample's y bitwise equal to cwfa_coupling_f8 on its row.
+ * samples >= 1 (1 = cwfa_coupling_f8); with samples > 1: inverse = 1, cx != NULL, sumsq = NULL, samples * chp8 * H * W < 2^31. */
+int cwfa_coupling_f8_samples(const void* b_c8, const void* w_packed, const float* bias, int N, int samples, int H, int W, int BN,
+                             int chp8, const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                             float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
+                             int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream);
+/* Split^-1 + IDWT of K >= 2 latent samples fused with their per-voxel mean and unbiased standard deviation (Welford): the K
+ * merged volumes are never written.  lo: K rows (B, C/2, P) or, lo_shared = 1, one row for every sample; hi: K rows in F8
+ * (hi_f8 = 1; P % 4 == 0, 16-byte aligned) or NCHW; mean, std: (C, P) each. */
+int cwfa_haar1d_inv_stats(const float* lo, int lo_shared, const float* hi, int hi_f8, float* mean, float* std, int K, int C,
+                          int64_t P, void* stream);
 /* Depth-wise Haar DWT + Split (INN_utils.py:142-161, graph_topology.py:73-80) with the detail half written / read in F8:
  * fwd: x (B,C,P) -> lo (B,C/2,P) NCHW, hi F8;  inv: lo, hi F8 -> x.  P % 4 == 0, pointers 16-byte aligned; every access 128-bit. */
 int cwfa_haar1d_fwd_f8(const float* x, float* lo, float* hi_f8, int B, int C, int64_t P, void* stream);
