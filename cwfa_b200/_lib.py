@@ -62,7 +62,7 @@ _SIGS = {
                               i32, vp, i32, vp],
     "cwfa_coupling_tc_tiles": [i32, i32],
     "cwfa_coupling_tc": [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, i32, f32, f32, i32, vp, vp, vp, i32, vp, i32, i32, i32, vp],
-    "cwfa_resblock_tc_batched": [vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, vp, i32, vp, i32, vp],
+    "cwfa_resblock_tc_batched": [vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, i32, i32, vp],
     "cwfa_coupling_finalize": [vp, vp, vp, i32, i32, i32, vp],
     "cwfa_coupling_f8": [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp, i32, i32, i32, vp],
     "cwfa_coupling_f8_samples": [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp,

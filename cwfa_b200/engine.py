@@ -76,9 +76,25 @@ class CWFAEngine:
                 batched = tc.PackedConv(torch.cat([w.weight.detach() for w in ws], 0), torch.cat([w.bias.detach() for w in ws], 0),
                                         kind, bn=64)
             self.levels.append(dict(nodes=nodes, cond=None if self.dlr else _CondNet(m.cond_nets[n], kind), batched_in=batched,
-                                    f8=self._plan_f8(nodes, kind)))
+                                    entry=self._plan_entry(nodes, kind), f8=self._plan_f8(nodes, kind)))
         self.lrnn = _LRNN(m.cond_nets[-1], kind)
         self._graphs: Dict = {}
+
+    @staticmethod
+    def _plan_entry(nodes, kind):
+        """The first trunk block of every fused sub-network folded onto its 1x1 input conv (``tc.PackedEntry``), or None when a
+        sub-network's input conv is not 1x1 Cin_p <= 64 -> 64, and for fp16.  fp16 keeps the separate input conv: its rounding
+        of W3' instead of Win and W3 moved the level-0 log-det of the full-size forward pass from 1.94e-3 to 2.24e-3 against the
+        fp32 reference (B200), past the fp16 engine's stated 2e-3."""
+        subs = [(mod.subnet, sn) for k, mod, sn in nodes if k == "cat"]
+        if kind != "bf16" or not subs or any(sn.inp.KH != 1 or sn.inp.Cout != 64 or sn.inp.Cin_p > 64
+                                             or sn.inp.Cin_p != subs[0][1].inp.Cin_p for _, sn in subs):
+            return None
+        out = []
+        for sub, sn in subs:
+            first = sub.block12 if sub.normal else sub.block1
+            out.append(tc.PackedEntry(first.weight, first.bias, sub.block2[0].weight, sub.block2[0].bias, sn.res[0][1], kind))
+        return out
 
     use_f8 = True          # lean coupling path on the F8 layout (csrc/coupling_f8.cu) for levels made of CAT blocks + permutations
 
@@ -111,6 +127,9 @@ class CWFAEngine:
 
     # -------------------------------------------------------------------------------------
     batch_trunks = True    # the block rows of a level's sub-network trunks as ONE launch each (cwfa_resblock_tc_batched)
+    # the first trunk block reads the LF condition directly (tc.PackedEntry): no 1x1 input-conv launch, its output never in HBM;
+    # CWFA_COMPOSED_ENTRY=0 keeps the input conv + block pair (A/B measurements)
+    composed_entry = __import__("os").environ.get("CWFA_COMPOSED_ENTRY", "1") == "1"
 
     def _trunks(self, n: int, lf8: tc.C8, allow_batched: bool = True):
         """The trunks of all fused sub-networks of level n from the level's LF condition (C8).  They depend on the conditions
@@ -118,9 +137,28 @@ class CWFAEngine:
         Items: (kind, module, executor, trunk output C8, chunk offset of this sub-network's 64-channel slice in it).
         With a batched input conv the three block rows of the (<= 5) trunks run as three launches over all sub-networks."""
         lv = self.levels[n]
-        b_all = tc.conv_tc(lf8, lv["batched_in"]) if lv["batched_in"] is not None else None
         subs = [extra for kind, _, extra in lv["nodes"] if kind == "cat"]
         out, k = [], 0
+        if lv["entry"] is not None and self.composed_entry:
+            b_all = None
+            if allow_batched and self.batch_trunks and 2 <= len(subs) <= 5:
+                b_all = tc.resblock_tc_entry_batched(lf8, lv["entry"])
+                for r in (1, 2):
+                    b_all = tc.resblock_tc_batched(b_all, [sn.res[r] for sn in subs])
+            for kind, mod, extra in lv["nodes"]:
+                if kind != "cat":
+                    out.append((kind, mod, extra, None, 0))
+                    continue
+                if b_all is not None:
+                    out.append(("cat", mod, extra, b_all, 8 * k))
+                else:
+                    b = tc.resblock_tc_entry_batched(lf8, [lv["entry"][k]])
+                    for p3, p1 in extra.res[1:]:
+                        b = tc.resblock_tc(b, p3, p1)
+                    out.append(("cat", mod, extra, b, 0))
+                k += 1
+            return out
+        b_all = tc.conv_tc(lf8, lv["batched_in"]) if lv["batched_in"] is not None else None
         if b_all is not None and allow_batched and self.batch_trunks and 2 <= len(subs) <= 5:
             for r in range(3):
                 b_all = tc.resblock_tc_batched(b_all, [sn.res[r] for sn in subs])

@@ -594,5 +594,59 @@ def resblock_tc_batched(x: C8, sets, in_chunk_offs=None) -> C8:
     b3, b1 = vps([s_[0].bias.data_ptr() for s_ in sets]), vps([s_[1].bias.data_ptr() for s_ in sets])
     io, oo = (C.c_int * n)(*offs), (C.c_int * n)(*[8 * k for k in range(n)])
     _lib.call("cwfa_resblock_tc_batched", x.data.data_ptr(), y.data.data_ptr(), n, w3, w1, b3, b1, x.N, x.H, x.W, x.Cp // 8, io,
-              n * 8, oo, x.is_bf16, _stream())
+              n * 8, oo, None, None, 0, x.is_bf16, _stream())
+    return y
+
+
+class PackedEntry:
+    """The first block of a sub-network trunk folded onto the trunk's 1x1 input conv ``b = Win * lf + bin`` (no activation
+    between them, networks.py:60-87), for ``resblock_tc_entry_batched``: ``W3 (*) b = (W3_tap Win) (*) lf + W3 (*) bin``.
+    Composed once in fp64, then rounded to ``kind``: the 3x3 conv W3' from the Cin condition channels, the interior bias
+    ``b3 + sum_tap W3_tap bin``, the acc2 bias ``b1 + bin`` and the per-edge-class sums of ``W3_tap bin`` over the taps that fall
+    outside the image (the network zero-pads b, not lf)."""
+
+    def __init__(self, w_in: torch.Tensor, b_in: torch.Tensor, w3: torch.Tensor, b3: torch.Tensor, p1: PackedConv, kind: str):
+        wi, bi = w_in.detach().double(), b_in.detach().double()
+        w3d = w3.detach().double()
+        if wi.shape[0] != 64 or wi.shape[2:] != (1, 1) or wi.shape[1] > 64 or tuple(w3d.shape) != (64, 64, 3, 3):
+            raise ValueError("PackedEntry: needs a 1x1 conv Cin (<= 64) -> 64 followed by a 3x3 conv 64 -> 64")
+        if p1.Cin_p != 64 or p1.Cout_p != 64 or p1.BN != 64 or p1.KH != 1 or p1.bias is None or p1.kind != kind:
+            raise ValueError("PackedEntry: needs the block's 1x1 conv 64 -> 64 packed with BN=64 and a bias")
+        comp = torch.einsum("omhw,mc->ochw", w3d, wi[:, :, 0, 0])
+        ctap = torch.einsum("omhw,m->hwo", w3d, bi)                           # W3_tap bin, (3, 3, 64)
+        edge = torch.zeros(4, 4, 64, device=ctap.device, dtype=torch.float64)
+        for r in range(4):                  # row class: bit 0 = first image row (kh = 0 out), bit 1 = last row (kh = 2 out)
+            for c in range(4):              # column class: bit 0 = first column (kw = 0 out), bit 1 = last column (kw = 2 out)
+                for kh in range(3):
+                    for kw in range(3):
+                        if (kh == 0 and r & 1) or (kh == 2 and r & 2) or (kw == 0 and c & 1) or (kw == 2 and c & 2):
+                            edge[r, c] += ctap[kh, kw]
+        self.kind, self.Cin = kind, wi.shape[1]
+        self.p3 = PackedConv(comp.float(), None, kind, bn=64)
+        self.pin = PackedConv(w_in, None, kind, bn=64)
+        self.p1 = p1
+        self.b3 = (b3.detach().double() + ctap.sum((0, 1))).float().contiguous()
+        self.b1 = (p1.bias.double() + bi).float().contiguous()
+        self.edge = edge.reshape(16, 64).float().contiguous()
+
+
+def resblock_tc_entry_batched(lf: C8, entries) -> C8:
+    """``ELU(W1 ELU(W3 (*) b + b3) + b1 + b)`` with ``b = Win lf + bin`` (zero-padded) for several sub-networks reading the same
+    LF condition ``lf``, in one ``cwfa_resblock_tc_batched`` launch of the entry form: ``entries`` = [PackedEntry, ...] (<= 5);
+    set k writes slice k of the returned tensor (64 * len(entries) channels).  b is never written."""
+    import ctypes as C
+    n = len(entries)
+    if not 1 <= n <= 5:
+        raise ValueError("resblock_tc_entry_batched: 1..5 weight sets")
+    if lf.Cp > 64 or any(e.p3.Cin_p != lf.Cp or e.kind != lf.kind for e in entries):
+        raise ValueError(f"resblock_tc_entry_batched: condition has Cp={lf.Cp}/{lf.kind}, the entry blocks expect another layout")
+    y = C8.empty(lf.N, 64 * n, lf.H, lf.W, lf.data.device, lf.kind, 64 * n)
+    vps = lambda vals: (C.c_void_p * n)(*vals)
+    w3, w1, win = (vps([e.p3.packed.data_ptr() for e in entries]), vps([e.p1.packed.data_ptr() for e in entries]),
+                   vps([e.pin.packed.data_ptr() for e in entries]))
+    b3, b1, edge = (vps([e.b3.data_ptr() for e in entries]), vps([e.b1.data_ptr() for e in entries]),
+                    vps([e.edge.data_ptr() for e in entries]))
+    io, oo = (C.c_int * n)(*([0] * n)), (C.c_int * n)(*[8 * k for k in range(n)])
+    _lib.call("cwfa_resblock_tc_batched", lf.data.data_ptr(), y.data.data_ptr(), n, w3, w1, b3, b1, lf.N, lf.H, lf.W, lf.Cp // 8, io,
+              n * 8, oo, win, edge, lf.Cp // 8, lf.is_bf16, _stream())
     return y

@@ -194,11 +194,18 @@ int cwfa_resblock_tc(const void* x_c8, void* y_c8, const void* w3_packed, const 
                      int in_chunk_off, int out_total_chunks, int out_chunk_off, int is_bf16, void* stream);
 /* The same block for n_sets (<= 5) independent sub-networks in ONE launch (the block row of a level's five coupling
  * sub-networks, networks.py:305-366): set k reads the slice at in_chunk_off[k] of x, writes the slice at out_chunk_off[k] of y,
- * with its own packed weights / biases (host arrays of n_sets pointers / offsets). */
+ * with its own packed weights / biases (host arrays of n_sets pointers / offsets).
+ * win_packed == NULL: the block above (edge and in_chunks are ignored).  Otherwise the ENTRY form, the first block of a trunk
+ * whose input b = Win * x + bin is the trunk's 1x1 input conv of the LF condition x: set k reads in_chunks (2, 4, 6 or 8) chunks
+ * of x at in_chunk_off[k] and computes y = ELU( W1 * ELU( W3 (*) b + b3 ) + b1 + b ) with b zero-padded, without b in memory.
+ * Per set: w3_packed = the composed 3x3 conv W3'_tap = W3_tap Win (cwfa_tc_pack_weights, Cin_p = 8 in_chunks, BN = 64),
+ * b3 = b3 + sum_tap W3_tap bin, b1 = b1 + bin, win_packed = Win (1x1, Cin_p = 8 in_chunks, BN = 64), edge = fp32 [16][64]:
+ * row (r * 4 + c) = sum of W3_tap bin over the taps outside the image for a pixel of row class r (bit 0: first image row,
+ * bit 1: last) and column class c (bit 0: first column, bit 1: last); all 16-byte aligned. */
 int cwfa_resblock_tc_batched(const void* x_c8, void* y_c8, int n_sets, const void* const* w3_packed,
                              const void* const* w1_packed, const float* const* b3, const float* const* b1, int N, int H, int W,
                              int in_total_chunks, const int* in_chunk_off, int out_total_chunks, const int* out_chunk_off,
-                             int is_bf16, void* stream);
+                             const void* const* win_packed, const float* const* edge, int in_chunks, int is_bf16, void* stream);
 /* ---- C8 helpers of the LRNN U-Net: per-channel (sum, sumsq) over (N,H,W) -> stats[2*Cp]
  * (workspace >= cwfa_c8_stats_workspace_floats(Cp) floats; feed to cwfa_bn_finalize_f32), and BatchNorm
  * apply y = x*scale+shift, optionally also writing the 2x2 max-pooled tensor (unet.py:79).

@@ -113,6 +113,12 @@ sets5 = [(tc.PackedConv(torch.randn(64, 64, 3, 3, device=DEV) * 0.04, torch.zero
           tc.PackedConv(torch.randn(64, 64, 1, 1, device=DEV) * 0.1, torch.zeros(64, device=DEV), bn=64)) for _ in range(5)]
 tensor("resblock_tc_batched: the block row of 5 sub-network trunks in one launch (5 x 64 ch) @512x512", 5 * 2.0 * P * 64 * 64 * 10, lambda i: tc.resblock_tc_batched(x5[i], sets5), 4)
 del x5
+lf48 = [tc.to_c8(torch.randn(1, 48, 512, 512, device=DEV)) for _ in range(4)]
+ent5 = [tc.PackedEntry(torch.randn(64, 48, 1, 1, device=DEV) * 0.14, torch.randn(64, device=DEV) * 0.1, torch.randn(64, 64, 3, 3, device=DEV) * 0.04, torch.zeros(64, device=DEV), sets5[k][1], "bf16") for k in range(5)]
+# algorithmic flops of the pair it replaces (1x1 conv 48 -> 64 + the block); the launch executes fewer: W3' has 48 input channels
+tensor("resblock_tc_entry_batched: 1x1 input conv folded into the first block, 5 trunks (48 -> 5 x 64) @512x512",
+       5 * 2.0 * P * (48 * 64 + 64 * 64 * 10), lambda i: tc.resblock_tc_entry_batched(lf48[i], ent5), 4)
+del lf48
 hx = [torch.randn(1, 96, 512, 512, device=DEV) for _ in range(4)]
 hbm("haar1d split, detail half in F8 (C=96)", 2 * 96 * P * 4, lambda i: tc.haar1d_split_f8(hx[i]), 4)
 lo4 = [torch.randn(1, 48, 512, 512, device=DEV) for _ in range(4)]
