@@ -311,14 +311,14 @@ __global__ void __launch_bounds__(256) c8_prelu_bwd_kernel(const uint4* __restri
     float s[8], q[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) s[j] = q[j] = 0.f;
-    // MODE 0: PReLU'(pre) = pre < 0 ? a : 1, q += dy * min(pre, 0).  MODE 1: ELU' from the OUTPUT y: y > 0 ? 1 : y + 1.
+    // MODE 0: PReLU'(pre) = pre > 0 ? 1 : a (torch's PReLU adjoint convention at pre = 0), q += dy * min(pre, 0).
+    // MODE 1: ELU' from the OUTPUT y: y > 0 ? 1 : y + 1.
     auto adj = [&](float (&dv)[8], const float (&pv)[8]) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             if constexpr (MODE == 0) {
-                const bool neg = pv[j] < 0.f;
-                q[j] = fmaf(dv[j], neg ? pv[j] : 0.f, q[j]);
-                dv[j] = neg ? a * dv[j] : dv[j];
+                q[j] = fmaf(dv[j], pv[j] < 0.f ? pv[j] : 0.f, q[j]);
+                dv[j] = pv[j] > 0.f ? dv[j] : a * dv[j];
             } else {
                 dv[j] *= pv[j] > 0.f ? 1.f : pv[j] + 1.f;
             }
