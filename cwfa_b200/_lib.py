@@ -67,6 +67,8 @@ _SIGS = {
     "cwfa_coupling_f8": [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp, i32, i32, i32, vp],
     "cwfa_coupling_f8_samples": [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp,
                                  i32, i32, i32, vp],
+    "cwfa_coupling_f8_map": [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp, i32, i32, i32,
+                             vp, vp, vp, vp, i32],
     "cwfa_haar1d_inv_stats": [vp, i32, vp, i32, vp, vp, i32, i32, i64, vp],
     "cwfa_haar1d_fwd_f8": [vp, vp, vp, i32, i32, i64, vp],
     "cwfa_haar1d_inv_f8": [vp, vp, vp, i32, i32, i64, vp],

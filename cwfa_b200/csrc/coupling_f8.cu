@@ -55,14 +55,22 @@ struct F8Params {
     int* ticket;
     int accumulate;
     int samples;                 // MS kernels: latent samples per condition image (x / y row n * samples + k)
+    float* map;                  // MAP kernels: F8 per-element NLL map, indexed by the element's coordinate at the level's input
+    const int* map_row;          //   R_b: input row of the element this block writes at output row h (NULL = identity)
+    const int* map_col;          //   C_b: the same for columns
+    int map_mode;                //   kMapFirst: write without reading; kMapLast: add 0.5 y^2 (both: a level of one block)
 };
+constexpr int kMapFirst = 1, kMapLast = 2;
 
 __device__ __forceinline__ float4 ldg128(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 
 // MS: the K-sample inverse variant (engine posterior statistics): one tile's accumulator, i.e. one evaluation of s and t,
 // serves the p.samples latent samples of its condition image.  MS = false is the frame path, unchanged.
-template <bool BF16, bool INV, bool EXT, bool MS = false>
+// MAP: the forward frame path that also accumulates each element's NLL term into p.map (see cwfa_coupling_f8_map); y, the
+// log-det and sum-of-squares partials are the MAP = false kernel's, instruction for instruction.
+template <bool BF16, bool INV, bool EXT, bool MS = false, bool MAP = false>
 __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_constant__ CUtensorMap tmap, const F8Params p) {
+    static_assert(!MAP || (!INV && !MS), "the NLL map is forward-only, one sample per condition image");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const uint32_t s0 = smem_u32(smem);
@@ -303,7 +311,12 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
             // coupling inputs of all of this thread's groups BEFORE the accumulator is ready (128-bit loads)
             float4 xv[kMaxG][2], tx[kMaxG][2];
             uint32_t ooff[kMaxG];                    // in-sample float offset of the output group
+            uint32_t moff[kMaxG];                    // MAP: in-sample float offset of the group's map entry (input coordinates)
             bool okg[kMaxG];
+            int mrow = orow;
+            if constexpr (MAP) {
+                if (row_ok && p.map_row) mrow = __ldg(p.map_row + orow);
+            }
 #pragma unroll
             for (int k = 0; k < kMaxG; ++k) {
                 const int g = sub + 4 * k;
@@ -317,6 +330,10 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                 const uint32_t gbase = (uint32_t)cg * plane;
                 ooff[k] = (gbase + (uint32_t)orow * (uint32_t)p.W + (uint32_t)ocol) * 8u;
                 const uint32_t soff = (gbase + (uint32_t)srow * (uint32_t)p.W + (uint32_t)scol) * 8u;
+                if constexpr (MAP) {
+                    const int mcol = (ok && p.map_col) ? __ldg(p.map_col + ocol) : ocol;
+                    moff[k] = (gbase + (uint32_t)mrow * (uint32_t)p.W + (uint32_t)mcol) * 8u;
+                }
                 const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (ok && has_x) {
                     xv[k][0] = ldg128(p.x + nbase + soff);
@@ -333,6 +350,17 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                     }
                 }
             }
+            // MAP: the running sums, one group ahead (those of all groups at once would not fit the register budget): group 0's
+            // before the accumulator wait, group k + 1's when group k starts.  EXT loads each group's when it starts: one group
+            // ahead spills there, and its block (the one with the external shift) is a level's first, which reads nothing.
+            float4 mnext[2];
+            auto map_load = [&](int k, float4* dst) {
+                const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+                const bool rd = okg[k] && !(p.map_mode & kMapFirst);
+                dst[0] = rd ? ldg128(p.map + nbase + moff[k]) : z4;
+                dst[1] = rd ? ldg128(p.map + nbase + moff[k] + 4) : z4;
+            };
+            if constexpr (MAP && !EXT) map_load(0, mnext);
             mbar_wait(acc_full(b), ph);
             tc_fence_after();
             float sum_a = 0.f, sum_q = 0.f;
@@ -341,6 +369,14 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                 const int g = sub + 4 * k;
                 if (g < ngroups) {                          // warp-uniform
                     const int mb = g >= gpc ? 1 : 0, cg = g - (mb ? gpc : 0);
+                    float4 m4[2];
+                    if constexpr (MAP && EXT) {
+                        map_load(k, m4);
+                    } else if constexpr (MAP) {
+                        m4[0] = mnext[0];
+                        m4[1] = mnext[1];
+                        if (k + 1 < kMaxG && g + 4 < ngroups) map_load(k + 1, mnext);
+                    }
                     uint32_t rs[8], rt[8];
                     __syncwarp();
                     const uint32_t ta = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * 256 + mb * p.BN + (cg << 3));
@@ -381,6 +417,19 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                         *reinterpret_cast<float4*>(yp + 4) = make_float4(yv[4], yv[5], yv[6], yv[7]);
                         sum_a += ga;
                         sum_q += gq;
+                        if constexpr (MAP) {
+                            // this block's term -s = -kk * atan(a_s) (the log-det's av, kk); the last block adds 0.5 y^2
+                            float mv[8] = {m4[0].x, m4[0].y, m4[0].z, m4[0].w, m4[1].x, m4[1].y, m4[1].z, m4[1].w};
+#pragma unroll
+                            for (int j = 0; j < 8; ++j) mv[j] = fmaf(-p.kk, av[j], mv[j]);
+                            if (p.map_mode & kMapLast) {
+#pragma unroll
+                                for (int j = 0; j < 8; ++j) mv[j] = fmaf(0.5f * yv[j], yv[j], mv[j]);
+                            }
+                            float* mp = p.map + nbase + moff[k];
+                            *reinterpret_cast<float4*>(mp) = make_float4(mv[0], mv[1], mv[2], mv[3]);
+                            *reinterpret_cast<float4*>(mp + 4) = make_float4(mv[4], mv[5], mv[6], mv[7]);
+                        }
                     }
                 }
             }
@@ -722,12 +771,15 @@ extern "C" int cwfa_f8_to_nchw(const float* x_f8, const int32_t* map, float* y, 
     return check_launch("f8_to_nchw");
 }
 
-// Shared launcher of cwfa_coupling_f8 (samples == 1) and cwfa_coupling_f8_samples.
+// Shared launcher of cwfa_coupling_f8 (samples == 1), cwfa_coupling_f8_samples and cwfa_coupling_f8_map (nll_map != NULL).
 static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_packed, const float* bias, int N, int samples, int H,
                               int W, int BN, int chp8, const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm,
                               int perm_axis, float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq,
-                              int accumulate, int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream) {
+                              int accumulate, int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream,
+                              float* nll_map = nullptr, const int32_t* row_src = nullptr, const int32_t* col_src = nullptr,
+                              int map_mode = 0) {
     const bool ms = samples > 1;
+    const bool map = nll_map != nullptr;
     if (samples < 1 || (ms && (!inverse || !cx || sumsq || (int64_t)samples * chp8 * H * W >= (1ll << 31)))) {
         set_error("%s: samples must be >= 1; with samples > 1 the coupling is inverse-only, needs x, has no sum of squares, and "
                   "samples * chp8 * H * W must stay below 2^31", name);
@@ -740,7 +792,7 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
         return CWFA_EINVAL;
     }
     if ((reinterpret_cast<uintptr_t>(b_c8) & 15) || (reinterpret_cast<uintptr_t>(w_packed) & 15) || !aligned16(cy) || (cx && !aligned16(cx)) ||
-        (ct && !aligned16(ct))) {
+        (ct && !aligned16(ct)) || (map && !aligned16(nll_map))) {
         set_error("%s: pointers must be 16-byte aligned", name);
         return CWFA_EINVAL;
     }
@@ -757,6 +809,7 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
     p.c2 = (inverse ? -kk : kk) * 1.4426950408889634f;
     p.tscale = t_scale;
     p.logdet = logdet; p.sumsq = sumsq; p.ticket = ticket; p.accumulate = accumulate; p.samples = samples;
+    p.map = nll_map; p.map_row = row_src; p.map_col = col_src; p.map_mode = map_mode;
     CUtensorMap tmap;
     p.in_chunk_off = in_chunk_off;
     int rc = make_c8_tensor_map(&tmap, b_c8, N, in_total_chunks, H, W, kBW, kBH, kChunks, is_bf16);
@@ -768,10 +821,13 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
     static const KernT table_ms[2][2] = {
         {coupling_f8_kernel<false, true, false, true>, coupling_f8_kernel<false, true, true, true>},
         {coupling_f8_kernel<true, true, false, true>, coupling_f8_kernel<true, true, true, true>}};
+    static const KernT table_map[2][2] = {
+        {coupling_f8_kernel<false, false, false, false, true>, coupling_f8_kernel<false, false, true, false, true>},
+        {coupling_f8_kernel<true, false, false, false, true>, coupling_f8_kernel<true, false, true, false, true>}};
     const int mode = (ct ? 2 : 0) + (inverse ? 1 : 0);
-    KernT kern = ms ? table_ms[is_bf16 ? 1 : 0][ct ? 1 : 0] : table[is_bf16 ? 1 : 0][mode];
-    static bool attr_done[12] = {false, false, false, false, false, false, false, false, false, false, false, false};
-    const int ki = ms ? 8 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : (is_bf16 ? 4 : 0) + mode;
+    KernT kern = ms ? table_ms[is_bf16 ? 1 : 0][ct ? 1 : 0] : map ? table_map[is_bf16 ? 1 : 0][ct ? 1 : 0] : table[is_bf16 ? 1 : 0][mode];
+    static bool attr_done[16] = {};
+    const int ki = ms ? 8 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : map ? 12 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : (is_bf16 ? 4 : 0) + mode;
     if (!attr_done[ki]) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         attr_done[ki] = true;
@@ -812,4 +868,26 @@ extern "C" int cwfa_coupling_f8_samples(const void* b_c8, const void* w_packed, 
     return coupling_f8_launch("coupling_f8_samples", b_c8, w_packed, bias, N, samples, H, W, BN, chp8, cx, cy, ct, t_scale, perm,
                               perm_axis, clamp, k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks,
                               in_chunk_off, is_bf16, stream);
+}
+// cwfa_coupling_f8 in the forward direction that also accumulates the per-element NLL terms of the level into nll_map (F8, the
+// layout of cx / cy).  Every coupling of a level is elementwise (s and t come from the conditions only), so each detail element
+// follows its own chain of affine maps and its NLL is 0.5 z^2 - sum over blocks of s.  nll_map is indexed by the element's
+// coordinate at the level's INPUT: this block adds its term at map[n, c, row_src[h], col_src[w]] for the element it writes at
+// (h, w) (row_src / col_src NULL = identity; the caller composes them from the level's row / column permutations; channels need
+// no table, F8 slots keep the order in which the detail half entered the flow).  map_mode: CWFA_NLL_MAP_FIRST writes -s without
+// reading nll_map (no memset needed), 0 (a middle block) adds -s, CWFA_NLL_MAP_LAST also adds 0.5 y^2 of the value it writes;
+// FIRST | LAST for a level of one block.  Padding slots come out 0.  cy, the log-det and sumsq are bitwise cwfa_coupling_f8's.
+// Rejected: inverse != 0, cx == NULL, nll_map == NULL, an unknown map_mode.
+extern "C" int cwfa_coupling_f8_map(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
+                                    const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                                    float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
+                                    int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream, float* nll_map,
+                                    const int32_t* row_src, const int32_t* col_src, int map_mode) {
+    if (inverse || !cx || !nll_map || map_mode < 0 || map_mode > (kMapFirst | kMapLast)) {
+        set_error("coupling_f8_map: forward only (inverse = 0), needs x and nll_map, map_mode in 0..3 (FIRST = 1 | LAST = 2)");
+        return CWFA_EINVAL;
+    }
+    return coupling_f8_launch("coupling_f8_map", b_c8, w_packed, bias, N, 1, H, W, BN, chp8, cx, cy, ct, t_scale, perm, perm_axis,
+                              clamp, k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks, in_chunk_off,
+                              is_bf16, stream, nll_map, row_src, col_src, map_mode);
 }

@@ -113,17 +113,48 @@ class CWFAEngine:
         dev = next(cats[0].parameters()).device
         m = torch.arange(ch)
         packed = []
+        # NLL maps (forward): (R_b, C_b) per CAT block in forward order = the level-input row / column of the element block b
+        # writes at (h, w).  A row / column permutation is gathered by the next coupling (y[h] = x[perm[h]]): R <- R[perm].
+        rc, src, pending = [None, None], [], None
         for k, mod, extra in nodes:
             if k == "perm" and extra == 1:
                 m = m[mod.perm.detach().cpu().long()]
+            elif k == "perm":
+                pending = (mod.perm.detach().cpu().long(), extra)
             elif k == "cat":
                 minv = torch.empty_like(m)
                 minv[m] = torch.arange(ch)
                 last = mod.subnet.block72[1] if mod.subnet.normal else mod.subnet.block7[1]
                 packed.append(tc.coupling_weights_f8(last.weight, last.bias, ch, minv, not mod.subnet.normal, kind))
+                if pending is not None:
+                    a = pending[1] - 2
+                    rc[a] = pending[0] if rc[a] is None else rc[a][pending[0]]
+                    pending = None
+                src.append(tuple(None if t is None else t.to(dev, torch.int32).contiguous() for t in rc))
         minv = torch.empty_like(m)
         minv[m] = torch.arange(ch)
-        return dict(ch=ch, out=packed, z_from_storage=m.to(dev, torch.int32).contiguous(), storage_from_z=minv.to(dev, torch.int32).contiguous())
+        return dict(ch=ch, out=packed, z_from_storage=m.to(dev, torch.int32).contiguous(), storage_from_z=minv.to(dev, torch.int32).contiguous(),
+                    map_src=src)
+
+    def _nll_map_unsupported(self, n: int, H: int, W: int) -> Optional[str]:
+        """Why level n has no per-voxel NLL map (maps come from the F8 coupling kernel), or None."""
+        lv = self.levels[n]
+        if lv["f8"] is not None and self.use_f8 and (H * W) % 4 == 0:
+            return None
+        if not self.use_f8:
+            return "the F8 coupling path is switched off (use_f8 = False)"
+        if lv["f8"] is not None:
+            return f"H * W = {H} * {W} is not a multiple of 4"
+        tanh = lambda mod: isinstance(mod, Fm.ConditionalAffineTransform) and bool(mod._clamp_kw and mod._clamp_kw["tanh_clamp"])
+        others = sorted({type(mod).__name__ + (" with a tanh clamp" if tanh(mod) else "") for k, mod, _ in lv["nodes"] if k == "module"})
+        if others:
+            return "its flow has blocks other than (non-tanh-clamped) ConditionalAffineTransform: " + ", ".join(others)
+        cats = [(mod, sub) for k, mod, sub in lv["nodes"] if k == "cat"]
+        if not cats:
+            return "its flow has no coupling block"
+        if cats[0][0].channels > 48:
+            return f"its detail half has {cats[0][0].channels} channels (at most 48)"
+        return "its coupling sub-networks are not 64 hidden channels with a 3x3 last conv"
 
     # -------------------------------------------------------------------------------------
     batch_trunks = True    # the block rows of a level's sub-network trunks as ONE launch each (cwfa_resblock_tc_batched)
@@ -262,10 +293,14 @@ class CWFAEngine:
             hi = ops.permute(hi, pending[0], pending[1])
         return hi, jac
 
-    def _couple_f8(self, item, pc, x8, mv8, pending, inverse, logdet, sumsq, ticket):
+    def _couple_f8(self, item, pc, x8, mv8, pending, inverse, logdet, sumsq, ticket, nll_map=None, map_src=(None, None), map_mode=0):
         _, mod, sub, b8, off = item
         first = not sub.normal
         perm, axis = (None, 0) if pending is None else (ops.perm_i32(pending[0], b8.data.device), pending[1])
+        if nll_map is not None:
+            return tc.coupling_f8_map(b8, pc, x8, nll_map, ch=mod.channels, map_mode=map_mode, row_src=map_src[0], col_src=map_src[1],
+                                      clamp=mod.clamp, t_ext8=mv8 if first else None, t_scale=(-1.0 / math.sqrt(2)) if first else 1.0,
+                                      perm=perm, perm_axis=axis, logdet=logdet, sumsq=sumsq, ticket=ticket, chunk_off=off)
         return tc.coupling_f8(b8, pc, x8, ch=mod.channels, inverse=inverse, clamp=mod.clamp, t_ext8=mv8 if first else None,
                               t_scale=(-1.0 / math.sqrt(2)) if first else 1.0, perm=perm, perm_axis=axis, logdet=logdet, sumsq=sumsq,
                               ticket=ticket, chunk_off=off)
@@ -502,27 +537,37 @@ class CWFAEngine:
         graph.replay()
         return out
 
-    def _level_forward_f8(self, n, plan, hi8, lf8, mean_vol):
+    def _level_forward_f8(self, n, plan, hi8, lf8, mean_vol, nll_map=False):
         ch = plan["ch"]
         jac, tickets = self._jac_and_tickets(hi8.shape[0], hi8.device)
         sumsq = torch.empty_like(jac)
         mv8 = None if mean_vol is None else tc.to_f8(mean_vol)
+        map8 = torch.empty_like(hi8) if nll_map else None        # the first coupling writes every entry: no memset
+        last = len(plan["out"]) - 1
         pending, k, ci = None, 0, 0
         for item in self._trunks(n, lf8):
             if item[0] == "cat":
-                hi8 = self._couple_f8(item, plan["out"][ci], hi8, mv8, pending, False, jac, sumsq, tickets[k:k + 1])   # sumsq: last coupling wins
+                if map8 is None:
+                    hi8 = self._couple_f8(item, plan["out"][ci], hi8, mv8, pending, False, jac, sumsq, tickets[k:k + 1])   # sumsq: last coupling wins
+                else:
+                    mode = (tc.NLL_MAP_FIRST if ci == 0 else 0) | (tc.NLL_MAP_LAST if ci == last else 0)
+                    hi8 = self._couple_f8(item, plan["out"][ci], hi8, mv8, pending, False, jac, sumsq, tickets[k:k + 1],
+                                          nll_map=map8, map_src=plan["map_src"][ci], map_mode=mode)
                 pending, k, ci = None, (k + 1) % tickets.numel(), ci + 1
             elif item[2] != 1:
                 pending = (item[1].perm, item[2])
         if pending is not None:
-            hi8 = self._permute_f8(hi8, ch, pending[0], pending[1])
-        return tc.from_f8(hi8, ch, plan["z_from_storage"]), jac, sumsq
+            hi8 = self._permute_f8(hi8, ch, pending[0], pending[1])     # moves z only: the map is in level-input coordinates
+        z = tc.from_f8(hi8, ch, plan["z_from_storage"])
+        if map8 is None:
+            return z, jac, sumsq
+        return z, jac, sumsq, tc.from_f8(map8, ch)
 
-    def _level_forward(self, n, hi, lf8, mean_vol):
-        """Detail half of level n through the flow in the forward direction: (z, logdet[B], sumsq[B]).  ``hi``: NCHW tensor, or
-        ("f8", tensor) from ``haar1d_split_f8`` for CAT-only levels."""
+    def _level_forward(self, n, hi, lf8, mean_vol, nll_map=False):
+        """Detail half of level n through the flow in the forward direction: (z, logdet[B], sumsq[B]), plus the (B, ch, H, W) NLL
+        map with ``nll_map`` (F8 levels only).  ``hi``: NCHW tensor, or ("f8", tensor) from ``haar1d_split_f8`` for CAT-only levels."""
         if isinstance(hi, tuple):
-            return self._level_forward_f8(n, self.levels[n]["f8"], hi[1], lf8, mean_vol)
+            return self._level_forward_f8(n, self.levels[n]["f8"], hi[1], lf8, mean_vol, nll_map)
         jac, tickets = self._jac_and_tickets(hi.shape[0], hi.device)
         sumsq = None
         pending, k, lf_nchw = None, 0, None
@@ -550,13 +595,22 @@ class CWFAEngine:
     @torch.no_grad()
     def forward_nll(self, volume: torch.Tensor, views: torch.Tensor, mean_vols: Sequence[torch.Tensor],
                     low_res_conditions: Optional[Sequence[torch.Tensor]] = None, _side_streams=None,
-                    sensor: Optional[LensletLayout] = None):
+                    sensor: Optional[LensletLayout] = None, nll_map: bool = False):
         """Forward pyramid + per-level NLL (CWFA.py:966-978); same outputs as CWFAModel.forward_nll.  ``sensor``: ``views`` is
         a raw sensor frame (see ``reconstruct``).
+
+        ``nll_map``: every level's dict also holds ``"nll_map"``, (B, ch, H, W) fp32: the NLL of each detail voxel,
+        0.5 z^2 - sum over the level's couplings of s, in the coordinates of the level's detail half (``haar1d_split(x)[1]``)
+        -- the couplings are elementwise, so this is exact, and ``nll_map.mean((1, 2, 3))`` is ``nll_per_sample``.  Channel c
+        of level n covers depths [c 2^(n+1), (c+1) 2^(n+1)) of the volume; ``.sum(1)`` is a lateral map.  Levels without the
+        F8 coupling plan (GLOW / RNVP / GIN / AI1 or tanh-clamped blocks, more than 48 detail channels, H * W not a multiple
+        of 4) raise ValueError.  z, the log-dets and the NLLs are bitwise those of ``nll_map=False``.
 
         The conditioning nets and trunks of the four levels depend on the views only, so under CUDA-graph capture
         (``forward_nll_graphed``) they run as parallel branches next to the Haar pyramid of the volume."""
         L1 = self.model.n_levels
+        if nll_map:
+            self._nll_map_check(volume)
         v8 = None if self.dlr else self._views_c8(views, sensor)
         # Haar pyramid of the volume first (cheap, sequential): lo_n / hi_n of every level
         los, his = [], []
@@ -575,8 +629,8 @@ class CWFAEngine:
             if self.dlr:
                 given = low_res_conditions[n] if low_res_conditions is not None and n < len(low_res_conditions) else None
                 lf8 = tc.to_c8(given if given is not None else los[n], self.kind)
-                return self._level_forward(n, his[n], lf8, None)
-            return self._level_forward(n, his[n], self._lf(n, v8, None), mean_vols[n])
+                return self._level_forward(n, his[n], lf8, None, nll_map)
+            return self._level_forward(n, his[n], self._lf(n, v8, None), mean_vols[n], nll_map)
 
         if _side_streams:
             main = torch.cuda.current_stream()
@@ -595,22 +649,36 @@ class CWFAEngine:
         else:
             results = [job(n) for n in range(L1)]
         res = []
-        for n, (z, jac, sumsq) in enumerate(results):
+        for n, r in enumerate(results):
+            z, jac, sumsq = r[:3]
             lo = los[n]
             per = (0.5 * sumsq - jac) / z[0].numel()
             ref = (0.5 * sumsq.sum() - jac) / lo.numel()
             res.append(dict(z=z, lo=lo, logdet=jac, sumsq=sumsq, nll_per_sample=per, nll_ref=ref))
+            if nll_map:
+                res[-1]["nll_map"] = r[3]
         return res
+
+    def _nll_map_check(self, volume: torch.Tensor):
+        for n in range(self.model.n_levels):
+            why = self._nll_map_unsupported(n, volume.shape[2], volume.shape[3])
+            if why is not None:
+                raise ValueError(f"forward_nll(nll_map=True): level {n} has no per-voxel NLL map: {why}")
 
     # ---- CUDA-graph replay of the forward pyramid (BASELINE.json configs[2]) ---------------------------------------------
     def forward_nll_graphed(self, volume: torch.Tensor, views: torch.Tensor, mean_vols: Sequence[torch.Tensor],
-                            sensor: Optional[LensletLayout] = None):
+                            sensor: Optional[LensletLayout] = None, nll_map: bool = False):
         """``forward_nll`` as one CUDA-graph replay (static shapes; inputs are copied into static buffers, the returned tensors
         are the graph's static outputs, overwritten by the next call): the four levels' conditioning nets / trunks / couplings
         are parallel branches of the graph.  ``sensor``: ``views`` is a raw sensor frame; the static input is the frame in its
-        own dtype and the lenslet extraction is part of the graph."""
+        own dtype and the lenslet extraction is part of the graph.  ``nll_map``: as in ``forward_nll``, a graph of its own whose
+        maps are static outputs too."""
+        if nll_map:
+            self._nll_map_check(volume)
         key = ("nll", tuple(volume.shape), tuple(views.shape), tuple(tuple(m.shape) for m in mean_vols), volume.device.index,
                None if sensor is None else (id(sensor), views.dtype))
+        if nll_map:
+            key = key + ("nll_map",)
         g = self._graphs.get(key)
         if g is None:
             sx, sv, sm = volume.clone(), views.clone(), [m.clone() for m in mean_vols]
@@ -618,12 +686,12 @@ class CWFAEngine:
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 for _ in range(2):
-                    self.forward_nll(sx, sv, sm, sensor=sensor)
+                    self.forward_nll(sx, sv, sm, sensor=sensor, nll_map=nll_map)
             torch.cuda.current_stream().wait_stream(s)
             graph = torch.cuda.CUDAGraph()
             side = [torch.cuda.Stream() for _ in range(self.model.n_levels)] if self.parallel_branches else None
             with torch.cuda.graph(graph):
-                out = self.forward_nll(sx, sv, sm, _side_streams=side, sensor=sensor)
+                out = self.forward_nll(sx, sv, sm, _side_streams=side, sensor=sensor, nll_map=nll_map)
             g = self._graphs[key] = (graph, sx, sv, sm, out, sensor)     # the graph reads the layout's coordinates: keep it alive
         graph, sx, sv, sm, out = g[:5]
         sx.copy_(volume, non_blocking=True)

@@ -530,6 +530,41 @@ def coupling_f8(b: C8, pc: PackedConv, x8: Optional[torch.Tensor], *, ch: int, i
     return y
 
 
+NLL_MAP_FIRST, NLL_MAP_LAST = 1, 2      # cwfa_coupling_f8_map's map_mode bits (include/cwfa_b200.h)
+
+
+def coupling_f8_map(b: C8, pc: PackedConv, x8: torch.Tensor, nll_map: torch.Tensor, *, ch: int, map_mode: int,
+                    row_src: Optional[torch.Tensor] = None, col_src: Optional[torch.Tensor] = None, clamp: float = 2.0,
+                    k_atan: float = 0.636, t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0,
+                    perm: Optional[torch.Tensor] = None, perm_axis: int = 0, logdet: torch.Tensor = None,
+                    sumsq: Optional[torch.Tensor] = None, accumulate: bool = True, ticket: Optional[torch.Tensor] = None,
+                    chunk_off: int = 0) -> torch.Tensor:
+    """Forward ``coupling_f8`` that also accumulates each element's NLL term into ``nll_map`` (F8, the shape of ``x8``), at the
+    element's coordinate at the level's input: ``(row_src[h], col_src[w])`` for the element written at ``(h, w)`` (int32 device
+    tables, None = identity).  ``map_mode``: ``NLL_MAP_FIRST`` writes -s without reading the map, 0 adds -s, ``NLL_MAP_LAST``
+    also adds 0.5 y^2.  The output, log-det and sumsq are bitwise ``coupling_f8``'s."""
+    if chunk_off * 8 + 64 > b.Cp or pc.Cin_p != 64 or pc.KH != 3 or pc.KW != 3 or b.kind != pc.kind or pc.BN != pc.Cout_p:
+        raise ValueError("coupling_f8_map: needs a 3x3 conv from 64 hidden channels packed in one n-block")
+    N, H, W = b.N, b.H, b.W
+    c8 = ch8(ch)
+    shape = (N, c8 // 8, H, W, 8)
+    if x8 is None or tuple(x8.shape) != shape or tuple(nll_map.shape) != shape or nll_map.dtype != torch.float32:
+        raise ValueError(f"coupling_f8_map: x8 and nll_map must be fp32 F8 tensors of shape {shape}")
+    for name, t, n_ in (("row_src", row_src, H), ("col_src", col_src, W)):
+        if t is not None and (t.dtype != torch.int32 or t.numel() != n_ or not t.is_cuda or not t.is_contiguous()):
+            raise ValueError(f"coupling_f8_map: {name} must be a contiguous int32 device tensor of {n_} entries")
+    y = torch.empty(shape, device=b.data.device, dtype=torch.float32)
+    tiles = _lib.load().cwfa_coupling_tc_tiles(H, W)
+    ws = torch.empty(2 * N * tiles, device=b.data.device, dtype=torch.float32)
+    _lib.call("cwfa_coupling_f8_map", b.data.data_ptr(), pc.packed.data_ptr(), _p(pc.bias), N, H, W, pc.BN, c8, x8.data_ptr(),
+              y.data_ptr(), _p(t_ext8), float(t_scale), _p(perm), int(perm_axis), float(clamp), float(k_atan), 0, ws.data_ptr(),
+              logdet.data_ptr(), _p(sumsq), int(accumulate), _p(ticket), b.Cp // 8, int(chunk_off), b.is_bf16, _stream(),
+              nll_map.data_ptr(), _p(row_src), _p(col_src), int(map_mode))
+    if ticket is None:
+        _lib.call("cwfa_coupling_finalize", ws.data_ptr(), logdet.data_ptr(), _p(sumsq), N, tiles, int(accumulate), _stream())
+    return y
+
+
 def coupling_f8_samples(b: C8, pc: PackedConv, x8: torch.Tensor, samples: int, *, ch: int, clamp: float = 2.0, k_atan: float = 0.636,
                         t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0, perm: Optional[torch.Tensor] = None,
                         perm_axis: int = 0, logdet: torch.Tensor = None, accumulate: bool = True,

@@ -305,6 +305,20 @@ int cwfa_coupling_f8_samples(const void* b_c8, const void* w_packed, const float
                              int chp8, const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
                              float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
                              int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream);
+/* cwfa_coupling_f8 in the forward direction (inverse = 0, cx != NULL) that also accumulates each detail element's NLL term into
+ * nll_map (F8, fp32, the layout of cx / cy): the couplings of a level are elementwise, so an element's NLL is 0.5 z^2 - sum of s
+ * over the level's blocks.  nll_map is indexed by the element's coordinate at the level's INPUT: the block adds -s (and, in the
+ * last block, 0.5 y^2) at [n][c / 8][row_src[h]][col_src[w]][c % 8] for the element it writes at (h, w); row_src / col_src are
+ * int32 tables composed from the level's row / column permutations (NULL = identity).  map_mode: CWFA_NLL_MAP_FIRST writes
+ * without reading nll_map, 0 adds to it, CWFA_NLL_MAP_LAST adds 0.5 y^2 too (FIRST | LAST for a level of one block).  Padding
+ * slots come out 0; cy, logdet and sumsq are bitwise those of cwfa_coupling_f8. */
+#define CWFA_NLL_MAP_FIRST 1
+#define CWFA_NLL_MAP_LAST 2
+int cwfa_coupling_f8_map(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
+                         const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                         float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
+                         int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream, float* nll_map,
+                         const int32_t* row_src, const int32_t* col_src, int map_mode);
 /* Split^-1 + IDWT of K >= 2 latent samples fused with their per-voxel mean and unbiased standard deviation (Welford): the K
  * merged volumes are never written.  lo: K rows (B, C/2, P) or, lo_shared = 1, one row for every sample; hi: K rows in F8
  * (hi_f8 = 1; P % 4 == 0, 16-byte aligned) or NCHW; mean, std: (C, P) each. */
