@@ -59,6 +59,8 @@ struct F8Params {
     const int* map_row;          //   R_b: input row of the element this block writes at output row h (NULL = identity)
     const int* map_col;          //   C_b: the same for columns
     int map_mode;                //   kMapFirst: write without reading; kMapLast: add 0.5 y^2 (both: a level of one block)
+    const float* scale_in;       // SCALE kernels: F8 d(x)/d(z) of the chain so far, gathered like x (NULL = 1)
+    float* scale_out;            //   F8 scale_in * exp(-s), written like y
 };
 constexpr int kMapFirst = 1, kMapLast = 2;
 
@@ -68,9 +70,13 @@ __device__ __forceinline__ float4 ldg128(const float* p) { return __ldg(reinterp
 // serves the p.samples latent samples of its condition image.  MS = false is the frame path, unchanged.
 // MAP: the forward frame path that also accumulates each element's NLL term into p.map (see cwfa_coupling_f8_map); y, the
 // log-det and sum-of-squares partials are the MAP = false kernel's, instruction for instruction.
-template <bool BF16, bool INV, bool EXT, bool MS = false, bool MAP = false>
+// SCALE: the inverse frame path that also carries each element's scale (the derivative of y by the level's latent) along the
+// chain: scale_out = scale_in * e with the factor e that y uses (see cwfa_coupling_f8_scale); y, the log-det and sum-of-squares
+// partials are the SCALE = false kernel's.
+template <bool BF16, bool INV, bool EXT, bool MS = false, bool MAP = false, bool SCALE = false>
 __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_constant__ CUtensorMap tmap, const F8Params p) {
     static_assert(!MAP || (!INV && !MS), "the NLL map is forward-only, one sample per condition image");
+    static_assert(!SCALE || (INV && !MS && !MAP), "the scale chain is inverse-only, one sample per condition image");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const uint32_t s0 = smem_u32(smem);
@@ -312,6 +318,7 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
             float4 xv[kMaxG][2], tx[kMaxG][2];
             uint32_t ooff[kMaxG];                    // in-sample float offset of the output group
             uint32_t moff[kMaxG];                    // MAP: in-sample float offset of the group's map entry (input coordinates)
+            uint32_t soffs[kMaxG];                   // SCALE: in-sample float offset of the group's gathered input
             bool okg[kMaxG];
             int mrow = orow;
             if constexpr (MAP) {
@@ -334,6 +341,7 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                     const int mcol = (ok && p.map_col) ? __ldg(p.map_col + ocol) : ocol;
                     moff[k] = (gbase + (uint32_t)mrow * (uint32_t)p.W + (uint32_t)mcol) * 8u;
                 }
+                if constexpr (SCALE) soffs[k] = soff;
                 const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (ok && has_x) {
                     xv[k][0] = ldg128(p.x + nbase + soff);
@@ -361,6 +369,16 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                 dst[1] = rd ? ldg128(p.map + nbase + moff[k] + 4) : z4;
             };
             if constexpr (MAP && !EXT) map_load(0, mnext);
+            // SCALE: the incoming scale one group ahead, as the map above (EXT: per group, one group ahead spills there); NULL
+            // scale_in (the chain's first block) reads nothing
+            float4 snext[2];
+            auto scale_load = [&](int k, float4* dst) {
+                const float4 one4 = make_float4(1.f, 1.f, 1.f, 1.f);
+                const bool rd = okg[k] && p.scale_in != nullptr;
+                dst[0] = rd ? ldg128(p.scale_in + nbase + soffs[k]) : one4;
+                dst[1] = rd ? ldg128(p.scale_in + nbase + soffs[k] + 4) : one4;
+            };
+            if constexpr (SCALE && !EXT) scale_load(0, snext);
             mbar_wait(acc_full(b), ph);
             tc_fence_after();
             float sum_a = 0.f, sum_q = 0.f;
@@ -377,6 +395,13 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                         m4[1] = mnext[1];
                         if (k + 1 < kMaxG && g + 4 < ngroups) map_load(k + 1, mnext);
                     }
+                    float si[8];
+                    if constexpr (SCALE) {
+                        if constexpr (EXT) scale_load(k, snext);
+                        si[0] = snext[0].x; si[1] = snext[0].y; si[2] = snext[0].z; si[3] = snext[0].w;
+                        si[4] = snext[1].x; si[5] = snext[1].y; si[6] = snext[1].z; si[7] = snext[1].w;
+                        if (!EXT && k + 1 < kMaxG && g + 4 < ngroups) scale_load(k + 1, snext);
+                    }
                     uint32_t rs[8], rt[8];
                     __syncwarp();
                     const uint32_t ta = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * 256 + mb * p.BN + (cg << 3));
@@ -389,7 +414,7 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                         te[0] = tx[k][0].x; te[1] = tx[k][0].y; te[2] = tx[k][0].z; te[3] = tx[k][0].w;
                         te[4] = tx[k][1].x; te[5] = tx[k][1].y; te[6] = tx[k][1].z; te[7] = tx[k][1].w;
                     }
-                    float yv[8], av[8];
+                    float yv[8], av[8], so[8];
 #pragma unroll
                     for (int j = 0; j < 8; ++j) av[j] = atan_fast(__uint_as_float(rs[j]));
 #pragma unroll
@@ -404,6 +429,7 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                         asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(p.c2 * av[j]));
                         if constexpr (INV) yv[j] = (xs[j] - tv) * e;
                         else yv[j] = fmaf(e, xs[j], tv);
+                        if constexpr (SCALE) so[j] = si[j] * e;
                     }
                     float ga = 0.f, gq = 0.f;
 #pragma unroll
@@ -417,6 +443,11 @@ __global__ void __launch_bounds__(kThreads, 1) coupling_f8_kernel(const __grid_c
                         *reinterpret_cast<float4*>(yp + 4) = make_float4(yv[4], yv[5], yv[6], yv[7]);
                         sum_a += ga;
                         sum_q += gq;
+                        if constexpr (SCALE) {
+                            float* sp = p.scale_out + nbase + ooff[k];
+                            *reinterpret_cast<float4*>(sp) = make_float4(so[0], so[1], so[2], so[3]);
+                            *reinterpret_cast<float4*>(sp + 4) = make_float4(so[4], so[5], so[6], so[7]);
+                        }
                         if constexpr (MAP) {
                             // this block's term -s = -kk * atan(a_s) (the log-det's av, kk); the last block adds 0.5 y^2
                             float mv[8] = {m4[0].x, m4[0].y, m4[0].z, m4[0].w, m4[1].x, m4[1].y, m4[1].z, m4[1].w};
@@ -556,6 +587,63 @@ __global__ void __launch_bounds__(256) haar1d_f8_kernel(const float* __restrict_
                 *reinterpret_cast<float4*>(hi_out + f8o + k * 8) = hv[k][0];
                 *reinterpret_cast<float4*>(hi_out + f8o + k * 8 + 4) = hv[k][1];
             }
+        }
+    }
+}
+
+// Split^-1 + IDWT of the z = 0 detail half fused with the exact standard-deviation rule of the merge.  The volume is affine in
+// the latents and the levels are independent, so with x[2i] = (lo_i + hi_i) / sqrt2 and x[2i+1] = (lo_i - hi_i) / sqrt2:
+// Var x[2i] = Var x[2i+1] = (Var lo_i + Var hi_i) / 2, Var hi_i = sigma^2 scale_i^2.  std_lo == NULL: lo is deterministic.
+// Same thread map as haar1d_f8_kernel; x is its INV expression, bit for bit.
+__global__ void __launch_bounds__(256) haar1d_inv_std_f8_kernel(const float* __restrict__ lo, const float* __restrict__ std_lo,
+                                                                const float* __restrict__ hi_in, const float* __restrict__ scale_in,
+                                                                float sigma, float* __restrict__ x, float* __restrict__ std_x,
+                                                                int B, int h, int64_t P) {
+    const int G = (h + 7) >> 3;
+    const int64_t P4 = P >> 2;
+    const int64_t total = (int64_t)B * G * P4;
+    for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t p4 = idx % P4;
+        const int64_t r = idx / P4;
+        const int g = (int)(r % G);
+        const int b = (int)(r / G);
+        const int64_t pix = p4 * 4;
+        float4 hv[4][2], sv[4][2];                         // [pixel][half of the group]
+        const int64_t f8o = (((int64_t)b * G + g) * P + pix) * 8;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            hv[k][0] = __ldg(reinterpret_cast<const float4*>(hi_in + f8o + k * 8));
+            hv[k][1] = __ldg(reinterpret_cast<const float4*>(hi_in + f8o + k * 8 + 4));
+            sv[k][0] = __ldg(reinterpret_cast<const float4*>(scale_in + f8o + k * 8));
+            sv[k][1] = __ldg(reinterpret_cast<const float4*>(scale_in + f8o + k * 8 + 4));
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int i = g * 8 + j;
+            if (i >= h) continue;                          // channel padding of the F8 group
+            const int64_t lo_o = ((int64_t)b * h + i) * P + pix;
+            const float4 l = __ldg(reinterpret_cast<const float4*>(lo + lo_o));
+            const float4 sl = std_lo ? __ldg(reinterpret_cast<const float4*>(std_lo + lo_o)) : make_float4(0.f, 0.f, 0.f, 0.f);
+            float hj[4], sj[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                hj[k] = reinterpret_cast<const float*>(&hv[k][j >> 2])[j & 3];
+                sj[k] = sigma * reinterpret_cast<const float*>(&sv[k][j >> 2])[j & 3];
+            }
+            float4 e, o, sd;
+            e.x = (l.x + hj[0]) * INV_SQRT2; o.x = (l.x - hj[0]) * INV_SQRT2;
+            e.y = (l.y + hj[1]) * INV_SQRT2; o.y = (l.y - hj[1]) * INV_SQRT2;
+            e.z = (l.z + hj[2]) * INV_SQRT2; o.z = (l.z - hj[2]) * INV_SQRT2;
+            e.w = (l.w + hj[3]) * INV_SQRT2; o.w = (l.w - hj[3]) * INV_SQRT2;
+            sd.x = __fsqrt_rn(0.5f * fmaf(sl.x, sl.x, sj[0] * sj[0]));
+            sd.y = __fsqrt_rn(0.5f * fmaf(sl.y, sl.y, sj[1] * sj[1]));
+            sd.z = __fsqrt_rn(0.5f * fmaf(sl.z, sl.z, sj[2] * sj[2]));
+            sd.w = __fsqrt_rn(0.5f * fmaf(sl.w, sl.w, sj[3] * sj[3]));
+            const int64_t xo = ((int64_t)b * 2 * h + 2 * i) * P + pix;
+            *reinterpret_cast<float4*>(x + xo) = e;
+            *reinterpret_cast<float4*>(x + xo + P) = o;
+            *reinterpret_cast<float4*>(std_x + xo) = sd;
+            *reinterpret_cast<float4*>(std_x + xo + P) = sd;
         }
     }
 }
@@ -741,6 +829,29 @@ extern "C" int cwfa_haar1d_inv_f8(const float* lo, const float* hi_f8, float* x,
     haar1d_f8_kernel<true><<<grid_for((int64_t)B * ((h + 7) / 8) * (P / 4)), 256, 0, (cudaStream_t)stream>>>(lo, hi_f8, x, nullptr, B, h, P);
     return check_launch("haar1d_inv_f8");
 }
+// cwfa_haar1d_inv_f8 fused with the exact standard deviation of the merged volume: see haar1d_inv_std_f8_kernel.  std_lo (the
+// shape of lo) NULL = 0; scale_f8 is the detail half's scale at unit latent variance (cwfa_coupling_f8_scale), sigma the
+// latents' standard deviation.  x is bitwise cwfa_haar1d_inv_f8's.
+extern "C" int cwfa_haar1d_inv_std_f8(const float* lo, const float* std_lo, const float* hi_f8, const float* scale_f8, float sigma,
+                                      float* x, float* std_x, int B, int C, int64_t P, void* stream) {
+    if (!(sigma >= 0.f && sigma <= 3.402823466e38f)) {      // also rejects NaN and +inf
+        set_error("haar1d_inv_std_f8: sigma must be finite and >= 0");
+        return CWFA_EINVAL;
+    }
+    if (!lo || !hi_f8 || !scale_f8 || !x || !std_x) {
+        set_error("haar1d_inv_std_f8: lo, hi_f8, scale_f8, x and std_x must not be NULL");
+        return CWFA_EINVAL;
+    }
+    if (B <= 0 || C <= 0 || (C & 1) || P <= 0 || (P & 3) || !aligned16(lo) || !aligned16(hi_f8) || !aligned16(scale_f8) || !aligned16(x) ||
+        !aligned16(std_x) || (std_lo && !aligned16(std_lo))) {
+        set_error("haar1d_inv_std_f8: needs even C, P %% 4 == 0 and 16-byte aligned pointers");
+        return CWFA_EINVAL;
+    }
+    const int h = C / 2;
+    haar1d_inv_std_f8_kernel<<<grid_for((int64_t)B * ((h + 7) / 8) * (P / 4)), 256, 0, (cudaStream_t)stream>>>(
+        lo, std_lo, hi_f8, scale_f8, sigma, x, std_x, B, h, P);
+    return check_launch("haar1d_inv_std_f8");
+}
 // Posterior statistics of the last merge: see haar1d_inv_stats_kernel.  lo: K rows (lo_shared = 0) or one row for all samples;
 // hi: K rows, F8 (hi_f8 = 1) or NCHW; mean / std: one (C, P) volume each.  F8 needs P % 4 == 0 and 16-byte aligned pointers;
 // NCHW uses 128-bit accesses when P % 4 == 0 and they are aligned, scalar ones otherwise.
@@ -771,15 +882,17 @@ extern "C" int cwfa_f8_to_nchw(const float* x_f8, const int32_t* map, float* y, 
     return check_launch("f8_to_nchw");
 }
 
-// Shared launcher of cwfa_coupling_f8 (samples == 1), cwfa_coupling_f8_samples and cwfa_coupling_f8_map (nll_map != NULL).
+// Shared launcher of cwfa_coupling_f8 (samples == 1), cwfa_coupling_f8_samples, cwfa_coupling_f8_map (nll_map != NULL) and
+// cwfa_coupling_f8_scale (scale_out != NULL).
 static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_packed, const float* bias, int N, int samples, int H,
                               int W, int BN, int chp8, const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm,
                               int perm_axis, float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq,
                               int accumulate, int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream,
                               float* nll_map = nullptr, const int32_t* row_src = nullptr, const int32_t* col_src = nullptr,
-                              int map_mode = 0) {
+                              int map_mode = 0, const float* scale_in = nullptr, float* scale_out = nullptr) {
     const bool ms = samples > 1;
     const bool map = nll_map != nullptr;
+    const bool scale = scale_out != nullptr;
     if (samples < 1 || (ms && (!inverse || !cx || sumsq || (int64_t)samples * chp8 * H * W >= (1ll << 31)))) {
         set_error("%s: samples must be >= 1; with samples > 1 the coupling is inverse-only, needs x, has no sum of squares, and "
                   "samples * chp8 * H * W must stay below 2^31", name);
@@ -792,7 +905,7 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
         return CWFA_EINVAL;
     }
     if ((reinterpret_cast<uintptr_t>(b_c8) & 15) || (reinterpret_cast<uintptr_t>(w_packed) & 15) || !aligned16(cy) || (cx && !aligned16(cx)) ||
-        (ct && !aligned16(ct)) || (map && !aligned16(nll_map))) {
+        (ct && !aligned16(ct)) || (map && !aligned16(nll_map)) || (scale && !aligned16(scale_out)) || (scale_in && !aligned16(scale_in))) {
         set_error("%s: pointers must be 16-byte aligned", name);
         return CWFA_EINVAL;
     }
@@ -810,6 +923,7 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
     p.tscale = t_scale;
     p.logdet = logdet; p.sumsq = sumsq; p.ticket = ticket; p.accumulate = accumulate; p.samples = samples;
     p.map = nll_map; p.map_row = row_src; p.map_col = col_src; p.map_mode = map_mode;
+    p.scale_in = scale_in; p.scale_out = scale_out;
     CUtensorMap tmap;
     p.in_chunk_off = in_chunk_off;
     int rc = make_c8_tensor_map(&tmap, b_c8, N, in_total_chunks, H, W, kBW, kBH, kChunks, is_bf16);
@@ -824,10 +938,15 @@ static int coupling_f8_launch(const char* name, const void* b_c8, const void* w_
     static const KernT table_map[2][2] = {
         {coupling_f8_kernel<false, false, false, false, true>, coupling_f8_kernel<false, false, true, false, true>},
         {coupling_f8_kernel<true, false, false, false, true>, coupling_f8_kernel<true, false, true, false, true>}};
+    static const KernT table_scale[2][2] = {
+        {coupling_f8_kernel<false, true, false, false, false, true>, coupling_f8_kernel<false, true, true, false, false, true>},
+        {coupling_f8_kernel<true, true, false, false, false, true>, coupling_f8_kernel<true, true, true, false, false, true>}};
     const int mode = (ct ? 2 : 0) + (inverse ? 1 : 0);
-    KernT kern = ms ? table_ms[is_bf16 ? 1 : 0][ct ? 1 : 0] : map ? table_map[is_bf16 ? 1 : 0][ct ? 1 : 0] : table[is_bf16 ? 1 : 0][mode];
-    static bool attr_done[16] = {};
-    const int ki = ms ? 8 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : map ? 12 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : (is_bf16 ? 4 : 0) + mode;
+    KernT kern = ms ? table_ms[is_bf16 ? 1 : 0][ct ? 1 : 0] : map ? table_map[is_bf16 ? 1 : 0][ct ? 1 : 0]
+               : scale ? table_scale[is_bf16 ? 1 : 0][ct ? 1 : 0] : table[is_bf16 ? 1 : 0][mode];
+    static bool attr_done[20] = {};
+    const int ki = ms ? 8 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : map ? 12 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0)
+                 : scale ? 16 + (is_bf16 ? 2 : 0) + (ct ? 1 : 0) : (is_bf16 ? 4 : 0) + mode;
     if (!attr_done[ki]) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         attr_done[ki] = true;
@@ -890,4 +1009,24 @@ extern "C" int cwfa_coupling_f8_map(const void* b_c8, const void* w_packed, cons
     return coupling_f8_launch("coupling_f8_map", b_c8, w_packed, bias, N, 1, H, W, BN, chp8, cx, cy, ct, t_scale, perm, perm_axis,
                               clamp, k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks, in_chunk_off,
                               is_bf16, stream, nll_map, row_src, col_src, map_mode);
+}
+// Inverse cwfa_coupling_f8 that also carries the scale of each detail element along the level's chain of couplings.  s and t come
+// from the conditions only, so y = (x - t) * exp(-s) is affine in x and a level's detail half is affine in its latent z:
+// hi[e] = beta[e] + alpha[e] * z[pi(e)], alpha = exp(-sum of the blocks' s).  scale_in (F8, the layout of cx; NULL = 1, the first
+// block in inverse order) is gathered through perm like cx; scale_out = scale_in * exp(-s) is written where cy is, with the
+// factor cy uses.  cy, the log-det and sumsq are bitwise cwfa_coupling_f8's.
+// Rejected: inverse == 0, scale_out == NULL, scale_out == scale_in (the gather makes in-place use a race).
+extern "C" int cwfa_coupling_f8_scale(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
+                                      const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                                      float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq,
+                                      int accumulate, int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream,
+                                      const float* scale_in, float* scale_out) {
+    if (!inverse || !scale_out || scale_out == scale_in) {
+        set_error("coupling_f8_scale: inverse only (inverse = 1), needs scale_out, and scale_out must not alias scale_in (the row / "
+                  "column gather reads other elements' scales)");
+        return CWFA_EINVAL;
+    }
+    return coupling_f8_launch("coupling_f8_scale", b_c8, w_packed, bias, N, 1, H, W, BN, chp8, cx, cy, ct, t_scale, perm, perm_axis,
+                              clamp, k_atan, inverse, workspace, logdet, sumsq, accumulate, ticket, in_total_chunks, in_chunk_off,
+                              is_bf16, stream, nullptr, nullptr, nullptr, 0, scale_in, scale_out);
 }

@@ -136,8 +136,9 @@ class CWFAEngine:
         return dict(ch=ch, out=packed, z_from_storage=m.to(dev, torch.int32).contiguous(), storage_from_z=minv.to(dev, torch.int32).contiguous(),
                     map_src=src)
 
-    def _nll_map_unsupported(self, n: int, H: int, W: int) -> Optional[str]:
-        """Why level n has no per-voxel NLL map (maps come from the F8 coupling kernel), or None."""
+    def _f8_unsupported(self, n: int, H: int, W: int) -> Optional[str]:
+        """Why level n does not run on the F8 coupling kernels (which give the per-voxel NLL maps and the exact posterior std),
+        or None."""
         lv = self.levels[n]
         if lv["f8"] is not None and self.use_f8 and (H * W) % 4 == 0:
             return None
@@ -293,10 +294,15 @@ class CWFAEngine:
             hi = ops.permute(hi, pending[0], pending[1])
         return hi, jac
 
-    def _couple_f8(self, item, pc, x8, mv8, pending, inverse, logdet, sumsq, ticket, nll_map=None, map_src=(None, None), map_mode=0):
+    def _couple_f8(self, item, pc, x8, mv8, pending, inverse, logdet, sumsq, ticket, nll_map=None, map_src=(None, None), map_mode=0,
+                   with_scale=False, scale8=None):
         _, mod, sub, b8, off = item
         first = not sub.normal
         perm, axis = (None, 0) if pending is None else (ops.perm_i32(pending[0], b8.data.device), pending[1])
+        if with_scale:
+            return tc.coupling_f8_scale(b8, pc, x8, scale8, ch=mod.channels, clamp=mod.clamp, t_ext8=mv8 if first else None,
+                                        t_scale=(-1.0 / math.sqrt(2)) if first else 1.0, perm=perm, perm_axis=axis, logdet=logdet,
+                                        ticket=ticket, chunk_off=off)
         if nll_map is not None:
             return tc.coupling_f8_map(b8, pc, x8, nll_map, ch=mod.channels, map_mode=map_mode, row_src=map_src[0], col_src=map_src[1],
                                       clamp=mod.clamp, t_ext8=mv8 if first else None, t_scale=(-1.0 / math.sqrt(2)) if first else 1.0,
@@ -310,8 +316,9 @@ class CWFAEngine:
         """Row / column permutation of an F8 tensor that no coupling follows (never the case in CWFA's graphs): via NCHW."""
         return tc.to_f8(ops.permute(tc.from_f8(x8, ch), perm, axis))
 
-    def _level_detail_inverse_f8(self, n, items, plan, lf8, mean_vol, z):
-        """Inverse of a CAT-only level on the F8 layout: returns (("f8", hi8), logdet)."""
+    def _level_detail_inverse_f8(self, n, items, plan, lf8, mean_vol, z, with_scale=False):
+        """Inverse of a CAT-only level on the F8 layout: returns (("f8", hi8), logdet).  ``with_scale``: the couplings also
+        carry each element's scale d hi / d z (``coupling_f8_scale``), returned as (("f8", hi8, scale8), logdet)."""
         ch = plan["ch"]
         hi = None if z is None else tc.to_f8(z, plan["storage_from_z"])
         mv8 = None if mean_vol is None else tc.to_f8(mean_vol)
@@ -319,16 +326,23 @@ class CWFAEngine:
         pending, k = None, 0
         pcs = plan["out"]
         ci = len(pcs)
+        sc = None                                               # scale of the chain so far; None = 1 (nothing gathered yet)
         for item in reversed(items):
             if item[0] == "cat":
                 ci -= 1
-                hi = self._couple_f8(item, pcs[ci], hi, mv8, pending, True, jac, None, tickets[k:k + 1])
+                if with_scale:
+                    hi, sc = self._couple_f8(item, pcs[ci], hi, mv8, pending, True, jac, None, tickets[k:k + 1], with_scale=True,
+                                             scale8=sc)
+                else:
+                    hi = self._couple_f8(item, pcs[ci], hi, mv8, pending, True, jac, None, tickets[k:k + 1])
                 pending, k = None, (k + 1) % tickets.numel()
             elif item[2] != 1 and hi is not None:               # row / column permutation: gathered by the next coupling
                 pending = (item[1].perm_inv, item[2])
         if pending is not None:
             hi = self._permute_f8(hi, ch, pending[0], pending[1])
-        return ("f8", hi), jac
+            if with_scale:
+                sc = self._permute_f8(sc, ch, pending[0], pending[1])
+        return (("f8", hi, sc) if with_scale else ("f8", hi)), jac
 
     @torch.no_grad()
     def reconstruct(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], return_all: bool = False,
@@ -444,10 +458,13 @@ class CWFAEngine:
             hi = self._permute_f8(hi, plan["ch"], pending[0], pending[1])
         return ("f8", hi)
 
-    def _posterior_check(self, views, n_samples, zs):
+    def _independent_levels_check(self):
         if self.dlr:
             raise ValueError("posterior statistics need independent levels: with disable_low_res_input each level is conditioned "
                              "on the volume reconstructed below it, so the samples are not a chain of independent levels")
+
+    def _posterior_check(self, views, n_samples, zs):
+        self._independent_levels_check()
         if int(n_samples) < 2:
             raise ValueError("posterior statistics need n_samples >= 2")
         if views.shape[0] != 1:
@@ -534,6 +551,87 @@ class CWFAEngine:
             if d is not None:
                 d.copy_(s_, non_blocking=True)
         self._fill_z(sz, zs, T)
+        graph.replay()
+        return out
+
+    # ---- exact posterior standard deviation: the volume is affine in the latents on CAT-only levels -------------------------
+    def _posterior_exact_sigma(self, temperature: Optional[float]) -> float:
+        """Checks that the exact moments exist for this model and returns sigma_T, the std of one latent at ``temperature``."""
+        from .pipeline import truncated_normal_var
+        self._independent_levels_check()
+        T = self.model.cfg.INN_z_temperature if temperature is None else temperature
+        var = truncated_normal_var(T)                             # ValueError for T < 0
+        for n in range(self.model.n_levels):
+            _, H, W = self.model.conv_inn[n].global_out_shapes[0]
+            why = self._f8_unsupported(n, H, W)
+            if why is not None:
+                raise ValueError(f"reconstruct_posterior_exact: level {n} has no exact posterior std: {why} (the exact moments "
+                                 "need every level affine in its latent: CAT blocks on the F8 coupling path)")
+        return math.sqrt(var)
+
+    @torch.no_grad()
+    def reconstruct_posterior_exact(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]],
+                                    temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None, _side_streams=None):
+        """Exact per-voxel posterior mean and standard deviation of the reconstruction under the latent prior, in one inverse
+        pass and for any batch size: ``(mean, std)``, each (B, D, H, W) fp32.
+
+        Every coupling of a level is a CAT block whose s and t come from the conditions only, so level n's detail half is affine in
+        its latent, hi_n = beta_n + alpha_n * z_n (alpha_n = exp(-sum of the blocks' s), carried along the chain by
+        ``coupling_f8_scale``); the levels are independent, the LRNN volume is deterministic and the Haar merge is linear.  Hence
+        mean = V(z = 0), bitwise ``reconstruct(views, mean_vols, temperature=0)``, and at every merge Var x[2i] = Var x[2i+1] =
+        (Var lo_i + Var hi_i) / 2 with Var hi_n = sigma_T^2 alpha_n^2, sigma_T^2 = ``truncated_normal_var(temperature)`` (default
+        ``cfg.INN_z_temperature``; 0 gives std = 0).  Only the mean and std are exact: a sum of scaled truncated normals is not
+        Gaussian.  ``reconstruct_posterior`` estimates the same two moments from K samples.
+
+        Raises ValueError for ``disable_low_res_input`` models (each level is conditioned on the volume below it, so the volume
+        is not affine in z), for levels without the F8 coupling plan (GLOW / RNVP / GIN / AI1 or tanh-clamped blocks, which are
+        not affine in z; more than 48 detail channels; H * W not a multiple of 4; ``use_f8 = False``) and for a negative
+        temperature.  ``sensor``: ``views`` is a raw sensor frame (see ``reconstruct``)."""
+        sigma = self._posterior_exact_sigma(temperature)
+        L1 = self.model.n_levels
+        v8 = self._views_c8(views, sensor)
+        mv_last = lrnn_mean_volume(mean_vols, L1)
+
+        def level(n):
+            lf8 = self._lf(n, v8, None)
+            return self._level_detail_inverse_f8(n, self._trunks(n, lf8), self.levels[n]["f8"], lf8, mean_vols[n], None, with_scale=True)
+
+        jobs = [lambda: self.lrnn(v8, mv_last)] + [(lambda n=n: level(n)) for n in range(L1 - 1, -1, -1)]
+        results = self._run_jobs(jobs, _side_streams)
+        vol, std = results[0], None                               # the LRNN volume is deterministic: std 0 (NULL)
+        for k in range(L1):
+            (_, hi8, sc8), _ = results[1 + k]
+            vol, std = tc.haar1d_merge_std_f8(vol, std, hi8, sc8, sigma)
+        return vol, std
+
+    def reconstruct_posterior_exact_graphed(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]],
+                                            temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None):
+        """``reconstruct_posterior_exact`` as one CUDA-graph replay, the LRNN and the levels as parallel branches.  sigma_T is a
+        kernel argument, so every temperature has a graph of its own.  The returned (mean, std) are the graph's static outputs,
+        overwritten by the next call with the same shapes and temperature."""
+        sigma = self._posterior_exact_sigma(temperature)
+        key = ("posterior_exact", tuple(views.shape), tuple(None if m is None else tuple(m.shape) for m in mean_vols), views.device.index,
+               sigma, None if sensor is None else (id(sensor), views.dtype))
+        g = self._graphs.get(key)
+        if g is None:
+            sv = views.clone()
+            sm = [None if m is None else m.clone() for m in mean_vols]
+            s = torch.cuda.Stream()
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                for _ in range(2):
+                    self.reconstruct_posterior_exact(sv, sm, temperature, sensor=sensor)
+            torch.cuda.current_stream().wait_stream(s)
+            graph = torch.cuda.CUDAGraph()
+            side = [torch.cuda.Stream() for _ in range(self.model.n_levels + 1)] if self.parallel_branches else None
+            with torch.cuda.graph(graph):
+                out = self.reconstruct_posterior_exact(sv, sm, temperature, sensor=sensor, _side_streams=side)
+            g = self._graphs[key] = (graph, sv, sm, out, sensor)    # the graph reads the layout's coordinates: keep it alive
+        graph, sv, sm, out = g[:4]
+        sv.copy_(views, non_blocking=True)
+        for d, s_ in zip(sm, mean_vols):
+            if d is not None:
+                d.copy_(s_, non_blocking=True)
         graph.replay()
         return out
 
@@ -661,7 +759,7 @@ class CWFAEngine:
 
     def _nll_map_check(self, volume: torch.Tensor):
         for n in range(self.model.n_levels):
-            why = self._nll_map_unsupported(n, volume.shape[2], volume.shape[3])
+            why = self._f8_unsupported(n, volume.shape[2], volume.shape[3])
             if why is not None:
                 raise ValueError(f"forward_nll(nll_map=True): level {n} has no per-voxel NLL map: {why}")
 

@@ -7,6 +7,7 @@ scope (SURVEY.md section 8).
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass, asdict
 from typing import List, Optional, Sequence
 
@@ -210,3 +211,14 @@ def sample_z_truncated(shape, device="cpu", temperature: float = 1.0) -> torch.T
     if temperature != 0:
         torch.nn.init.trunc_normal_(z, mean=0.0, std=1.0, a=-temperature, b=temperature)
     return z
+
+
+def truncated_normal_var(temperature: float) -> float:
+    """Variance of one ``sample_z_truncated`` draw: a unit normal truncated to [-T, T], 1 - 2 T phi(T) / (2 Phi(T) - 1), in double
+    precision; 0 at T = 0 (z = 0).  sigma_T = 0.39105 at T = 0.7."""
+    T = float(temperature)
+    if not (T >= 0.0 and math.isfinite(T)):
+        raise ValueError(f"temperature must be finite and >= 0, got {temperature}")
+    if T < 1e-3:
+        return T * T / 3.0 * (1.0 - 2.0 * T * T / 15.0)      # series: the closed form cancels to nothing as T -> 0
+    return 1.0 - 2.0 * T * math.exp(-0.5 * T * T) / math.sqrt(2.0 * math.pi) / math.erf(T / math.sqrt(2.0))

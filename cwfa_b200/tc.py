@@ -565,6 +565,54 @@ def coupling_f8_map(b: C8, pc: PackedConv, x8: torch.Tensor, nll_map: torch.Tens
     return y
 
 
+def coupling_f8_scale(b: C8, pc: PackedConv, x8: Optional[torch.Tensor], scale8: Optional[torch.Tensor], *, ch: int,
+                      clamp: float = 2.0, k_atan: float = 0.636, t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0,
+                      perm: Optional[torch.Tensor] = None, perm_axis: int = 0, logdet: torch.Tensor = None, accumulate: bool = True,
+                      ticket: Optional[torch.Tensor] = None, chunk_off: int = 0):
+    """Inverse ``coupling_f8`` that also carries the scale of every detail element along the level's chain: returns
+    ``(y8, scale_out)`` with ``scale_out = scale8 * exp(-s)``, ``scale8`` gathered through ``perm`` like ``x8`` (None = 1, the
+    chain's first block).  ``y8`` and the log-det are bitwise ``coupling_f8``'s."""
+    if chunk_off * 8 + 64 > b.Cp or pc.Cin_p != 64 or pc.KH != 3 or pc.KW != 3 or b.kind != pc.kind or pc.BN != pc.Cout_p:
+        raise ValueError("coupling_f8_scale: needs a 3x3 conv from 64 hidden channels packed in one n-block")
+    N, H, W = b.N, b.H, b.W
+    c8 = ch8(ch)
+    shape = (N, c8 // 8, H, W, 8)
+    for name, t in (("x8", x8), ("scale8", scale8)):
+        if t is not None and (tuple(t.shape) != shape or t.dtype != torch.float32):
+            raise ValueError(f"coupling_f8_scale: {name} must be an fp32 F8 tensor of shape {shape}")
+    y = torch.empty(shape, device=b.data.device, dtype=torch.float32)
+    s_out = torch.empty_like(y)
+    tiles = _lib.load().cwfa_coupling_tc_tiles(H, W)
+    ws = torch.empty(2 * N * tiles, device=b.data.device, dtype=torch.float32)
+    _lib.call("cwfa_coupling_f8_scale", b.data.data_ptr(), pc.packed.data_ptr(), _p(pc.bias), N, H, W, pc.BN, c8, _p(x8), y.data_ptr(),
+              _p(t_ext8), float(t_scale), _p(perm), int(perm_axis), float(clamp), float(k_atan), 1, ws.data_ptr(), logdet.data_ptr(),
+              None, int(accumulate), _p(ticket), b.Cp // 8, int(chunk_off), b.is_bf16, _stream(), _p(scale8), s_out.data_ptr())
+    if ticket is None:
+        _lib.call("cwfa_coupling_finalize", ws.data_ptr(), logdet.data_ptr(), None, N, tiles, int(accumulate), _stream())
+    return y, s_out
+
+
+def haar1d_merge_std_f8(lo: torch.Tensor, std_lo: Optional[torch.Tensor], hi8: torch.Tensor, scale8: torch.Tensor, sigma: float):
+    """``haar1d_merge_f8`` fused with the exact standard deviation of the merged volume: the detail half is
+    ``hi8 + sigma * scale8 * z`` (independent unit-variance z) and ``lo`` has the independent std ``std_lo`` (None = 0).  Returns
+    ``(x, std_x)``, (B, 2h, H, W) each; x is bitwise ``haar1d_merge_f8(lo, hi8)``, std_x[2i] = std_x[2i+1] =
+    sqrt((std_lo_i^2 + sigma^2 scale_i^2) / 2)."""
+    lo = _ck(lo, "lo")
+    B, h, H, W = lo.shape
+    want = (B, ch8(h) // 8, H, W, 8)
+    if tuple(hi8.shape) != want or tuple(scale8.shape) != want:
+        raise ValueError(f"haar1d_merge_std_f8: detail half {tuple(hi8.shape)} / scale {tuple(scale8.shape)}, expected {want}")
+    if std_lo is not None:
+        std_lo = _ck(std_lo, "std_lo")
+        if std_lo.shape != lo.shape:
+            raise ValueError(f"haar1d_merge_std_f8: std_lo has shape {tuple(std_lo.shape)}, expected {tuple(lo.shape)}")
+    x = torch.empty((B, 2 * h, H, W), device=lo.device, dtype=torch.float32)
+    std_x = torch.empty_like(x)
+    _lib.call("cwfa_haar1d_inv_std_f8", lo.data_ptr(), _p(std_lo), hi8.data_ptr(), scale8.data_ptr(), float(sigma), x.data_ptr(),
+              std_x.data_ptr(), B, 2 * h, H * W, _stream())
+    return x, std_x
+
+
 def coupling_f8_samples(b: C8, pc: PackedConv, x8: torch.Tensor, samples: int, *, ch: int, clamp: float = 2.0, k_atan: float = 0.636,
                         t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0, perm: Optional[torch.Tensor] = None,
                         perm_axis: int = 0, logdet: torch.Tensor = None, accumulate: bool = True,

@@ -319,6 +319,22 @@ int cwfa_coupling_f8_map(const void* b_c8, const void* w_packed, const float* bi
                          float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
                          int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream, float* nll_map,
                          const int32_t* row_src, const int32_t* col_src, int map_mode);
+/* cwfa_coupling_f8 in the inverse direction (inverse = 1) that also carries each detail element's scale along the level's chain
+ * of couplings: s and t come from the conditions only, so a level's detail half is affine in its latent, hi = beta + alpha * z
+ * with alpha = exp(-sum of the blocks' s).  scale_in (F8, fp32, the layout of cx; NULL = 1, the first block in inverse order) is
+ * gathered through perm like cx; scale_out = scale_in * exp(-s) is written where cy is.  cy, logdet and sumsq are bitwise those
+ * of cwfa_coupling_f8.  Rejected: inverse == 0, scale_out == NULL, scale_out == scale_in (in-place use races with the gather). */
+int cwfa_coupling_f8_scale(const void* b_c8, const void* w_packed, const float* bias, int N, int H, int W, int BN, int chp8,
+                           const float* cx, float* cy, const float* ct, float t_scale, const int32_t* perm, int perm_axis,
+                           float clamp, float k_atan, int inverse, float* workspace, float* logdet, float* sumsq, int accumulate,
+                           int32_t* ticket, int in_total_chunks, int in_chunk_off, int is_bf16, void* stream,
+                           const float* scale_in, float* scale_out);
+/* cwfa_haar1d_inv_f8 fused with the exact per-voxel standard deviation of the merged volume when the detail half is
+ * hi + sigma * scale * z with independent unit-variance latents z and lo carries the independent std std_lo (NULL = 0):
+ * std_x[2i] = std_x[2i+1] = sqrt(0.5 (std_lo_i^2 + sigma^2 scale_i^2)), correctly rounded sqrt.  x is bitwise cwfa_haar1d_inv_f8's.
+ * Rejected: sigma < 0 or not finite, a NULL lo / hi_f8 / scale_f8 / x / std_x, odd C, P % 4 != 0, unaligned pointers. */
+int cwfa_haar1d_inv_std_f8(const float* lo, const float* std_lo, const float* hi_f8, const float* scale_f8, float sigma, float* x,
+                           float* std_x, int B, int C, int64_t P, void* stream);
 /* Split^-1 + IDWT of K >= 2 latent samples fused with their per-voxel mean and unbiased standard deviation (Welford): the K
  * merged volumes are never written.  lo: K rows (B, C/2, P) or, lo_shared = 1, one row for every sample; hi: K rows in F8
  * (hi_f8 = 1; P % 4 == 0, 16-byte aligned) or NCHW; mean, std: (C, P) each. */
