@@ -8,7 +8,7 @@ Drop-in surface (same names / signatures / state_dict keys as the reference, pvj
 All arithmetic runs in hand-written CUDA kernels behind the C ABI in include/cwfa_b200.h.
 """
 from . import _lib, data, framework, modules, networks, ops, packed  # noqa: F401
-from .data import LensletLayout  # noqa: F401
+from .data import LensletLayout, RoiSet  # noqa: F401
 from .packed import inference_precision, set_inference_precision, weights_changed  # noqa: F401
 from .pipeline import CWFAModel, CWFAConfig  # noqa: F401
 

@@ -72,6 +72,7 @@ _SIGS = {
     "cwfa_coupling_f8_scale": [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, f32, vp, i32, f32, f32, i32, vp, vp, vp, i32, vp, i32, i32,
                                i32, vp, vp, vp],
     "cwfa_haar1d_inv_std_f8": [vp, vp, vp, vp, f32, vp, vp, i32, i32, i64, vp],
+    "cwfa_roi_readout_f8": [vp, i64, vp, vp, i32, vp, vp, vp, vp, vp, vp, i32, i32, f32, vp, vp, vp],
     "cwfa_haar1d_inv_stats": [vp, i32, vp, i32, vp, vp, i32, i32, i64, vp],
     "cwfa_haar1d_fwd_f8": [vp, vp, vp, i32, i32, i64, vp],
     "cwfa_haar1d_inv_f8": [vp, vp, vp, i32, i32, i64, vp],

@@ -117,6 +117,140 @@ class LensletLayout:
         return out
 
 
+_ROI_MAX_LEVELS = 8                      # the readout kernel's per-level pointer table (cwfa_roi_readout_f8)
+
+
+def _roi_csr(roi: torch.Tensor, off: torch.Tensor, plus: torch.Tensor, minus: torch.Tensor, size: int, n_rois: int, scale: float):
+    """CSR over ROIs of ``(offset, scale * (sum of plus - sum of minus))`` per distinct (roi, offset), entries of an ROI sorted
+    by offset, exact zeros dropped.  The two sums are accumulated apart in float64 (index_add_ on the CPU, in entry order), so
+    equal weights on both halves of a Haar block cancel to exactly 0 instead of to a rounding residue."""
+    key = roi * size + off
+    uniq, inv = torch.unique(key, sorted=True, return_inverse=True)
+    p = torch.zeros(uniq.numel(), dtype=torch.float64).index_add_(0, inv, plus)
+    m = torch.zeros(uniq.numel(), dtype=torch.float64).index_add_(0, inv, minus)
+    val = (p - m) * scale
+    keep = val != 0
+    uniq, val = uniq[keep], val[keep]
+    ptr = torch.zeros(n_rois + 1, dtype=torch.int64)
+    ptr[1:] = torch.cumsum(torch.bincount(uniq // size, minlength=n_rois), 0)
+    return ptr, (uniq % size).to(torch.int32), val.to(torch.float32)
+
+
+def roi_tables(roi, voxel, weight, n_rois: int, volume_shape: Sequence[int], n_levels: int) -> Dict[str, torch.Tensor]:
+    """The readout tables of ``RoiSet`` from COO triplets, in pure torch on the CPU (float64 sums, fp32 storage).
+
+    ROI r reads ``r = sum_v w_v V[d_v, h_v, w_v]`` over its triplets ``(roi = r, voxel = (d, h, w), weight = w)``; repeated
+    voxels add up.  Returns
+
+      * ``mean_ptr`` (R + 1,) int64, ``mean_idx`` int32, ``mean_w`` fp32: a CSR over ROIs of (offset ``(d H + h) W + w`` into one
+        (D, H, W) volume, summed weight);
+      * ``coef_ptr`` (L, R + 1) int64, ``coef_idx`` int32, ``coef_val`` fp32: per level n a CSR over ROIs, with offsets into the
+        shared ``coef_idx`` / ``coef_val`` (level n's entries follow level n - 1's), of (offset into level n's F8 scale tensor of one
+        batch item, ``((i >> 3) H W + h W + w) 8 + (i & 7)``, coefficient ``w~_n[i, h, w]``).  ``w~_n`` is level n's detail half
+        of the forward depth Haar analysis of the weight volume (``oracle.cwfa_oracle.haar1d``, applied n + 1 times):
+        ``w~_n[i, h, w] = 2^(-(n+1)/2) (sum of w[d, h, w] over the first half of depths [i 2^(n+1), (i+1) 2^(n+1)) - sum over
+        the second half)``.
+
+    Within an ROI the entries are sorted by offset; entries that are exactly 0 are dropped.  Raises ValueError for voxels out of
+    range, non-finite weights, ``roi`` outside [0, n_rois), ``n_rois < 1``, ``n_levels`` outside 1..8, and D not divisible by
+    2^n_levels."""
+    n_rois, n_levels = int(n_rois), int(n_levels)
+    if n_rois < 1:
+        raise ValueError(f"n_rois must be >= 1, got {n_rois}")
+    if not 1 <= n_levels <= _ROI_MAX_LEVELS:
+        raise ValueError(f"n_levels must be in 1..{_ROI_MAX_LEVELS}, got {n_levels}")
+    if len(volume_shape) != 3 or any(int(s) < 1 for s in volume_shape):
+        raise ValueError(f"volume_shape must be three positive sizes (D, H, W), got {tuple(volume_shape)}")
+    D, H, W = (int(s) for s in volume_shape)
+    if D % (1 << n_levels):
+        raise ValueError(f"D = {D} is not divisible by 2^n_levels = {1 << n_levels}")
+    if D * H * W >= 2 ** 31 or ((D // 2 + 7) // 8) * 8 * H * W >= 2 ** 31:
+        raise ValueError(f"volume {D}x{H}x{W} is too large for the tables' int32 offsets")
+    roi, voxel, weight = (torch.as_tensor(t).detach().cpu() for t in (roi, voxel, weight))
+    if roi.is_floating_point() or roi.is_complex() or roi.dtype == torch.bool or roi.dim() != 1:
+        raise ValueError(f"roi must be a 1-D integer array, got {roi.dtype} of shape {tuple(roi.shape)}")
+    if voxel.is_floating_point() or voxel.is_complex() or voxel.dtype == torch.bool or voxel.dim() != 2 or voxel.shape[1] != 3:
+        raise ValueError(f"voxel must be an (N, 3) integer array of (d, h, w), got {voxel.dtype} of shape {tuple(voxel.shape)}")
+    if not (weight.is_floating_point() or weight.dtype in (torch.int32, torch.int64)) or weight.dim() != 1:
+        raise ValueError(f"weight must be a 1-D float array, got {weight.dtype} of shape {tuple(weight.shape)}")
+    if not roi.shape[0] == voxel.shape[0] == weight.shape[0]:
+        raise ValueError(f"roi, voxel and weight have {roi.shape[0]}, {voxel.shape[0]} and {weight.shape[0]} entries")
+    roi, voxel, wt = roi.long(), voxel.long(), weight.double()
+    if roi.numel() and (int(roi.min()) < 0 or int(roi.max()) >= n_rois):
+        raise ValueError(f"roi indices must lie in [0, {n_rois})")
+    d, h, w = voxel.unbind(1)
+    for name, a, n in (("d", d, D), ("h", h, H), ("w", w, W)):
+        if a.numel() and (int(a.min()) < 0 or int(a.max()) >= n):
+            raise ValueError(f"voxel {name} index out of range [0, {n})")
+    if not bool(torch.isfinite(wt).all()):
+        raise ValueError("weights must be finite")
+    zero = torch.zeros_like(wt)
+    mean_ptr, mean_idx, mean_w = _roi_csr(roi, (d * H + h) * W + w, wt, zero, D * H * W, n_rois, 1.0)
+    ptrs, idxs, vals, base = [], [], [], 0
+    for n in range(n_levels):
+        i = d >> (n + 1)
+        first = ((d >> n) & 1) == 0                             # first half of the 2^(n+1)-plane block of element i
+        size = ((D // 2 ** (n + 1) + 7) // 8) * 8 * H * W       # one batch item of level n's F8 tensor
+        off = ((i >> 3) * (H * W) + h * W + w) * 8 + (i & 7)
+        ptr, idx, val = _roi_csr(roi, off, torch.where(first, wt, zero), torch.where(first, zero, wt), size, n_rois,
+                                 2.0 ** (-(n + 1) / 2))
+        ptrs.append(ptr + base)
+        idxs.append(idx)
+        vals.append(val)
+        base += idx.numel()
+    return dict(mean_ptr=mean_ptr, mean_idx=mean_idx, mean_w=mean_w, coef_ptr=torch.stack(ptrs),
+                coef_idx=torch.cat(idxs), coef_val=torch.cat(vals))
+
+
+class RoiSet:
+    """Region readouts of a reconstructed volume, e.g. neuron footprints, held on the device once per recording:
+    ``rois = RoiSet.from_labels(labels, n_levels)``, then per frame ``engine.roi_posterior_exact_graphed(views, mean_vols, rois)``
+    gives each ROI's posterior mean and exact standard deviation.
+
+    ``RoiSet(roi, voxel, weight, n_rois, volume_shape=(D, H, W), n_levels=L)``: COO triplets; ROI r reads
+    ``sum_v w_v V[d_v, h_v, w_v]`` (soft footprints and overlapping ROIs are fine; repeated voxels add up).  ``n_levels`` is the
+    model's number of flow levels.  The tables (``roi_tables``: the weights, and per level the Haar detail coefficients of the
+    weight volume at the offsets of the engine's F8 scale tensors) are built on the CPU in float64, so they are the same on
+    every run, then copied to ``device``.  An ROI without voxels reads 0 with std 0."""
+
+    def __init__(self, roi, voxel, weight, n_rois: int, volume_shape: Sequence[int], n_levels: int, device="cuda"):
+        t = roi_tables(roi, voxel, weight, n_rois, volume_shape, n_levels)
+        self.n_rois, self.n_levels = int(n_rois), int(n_levels)
+        self.volume_shape: Tuple[int, int, int] = tuple(int(s) for s in volume_shape)
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        self.device = device
+        self.n_mean_entries, self.n_coef_entries = int(t["mean_idx"].numel()), int(t["coef_idx"].numel())
+        for k, v in t.items():
+            if v.numel() == 0:                  # the kernel takes non-NULL pointers; no ptr range ever reaches this element
+                v = torch.zeros(1, dtype=v.dtype)
+            setattr(self, k, v.to(device).contiguous())
+
+    @classmethod
+    def from_labels(cls, labels, n_levels: int, device="cuda") -> "RoiSet":
+        """ROIs from a (D, H, W) integer label volume: 0 is background, ROI r is label r + 1 and reads the mean over its voxels
+        (weight 1 / |r|).  ``n_rois`` is the largest label; a label value that no voxel carries is an empty ROI."""
+        lab = torch.as_tensor(labels).detach().cpu()
+        if lab.is_floating_point() or lab.is_complex() or lab.dtype == torch.bool or lab.dim() != 3:
+            raise ValueError(f"labels must be a (D, H, W) integer volume, got {lab.dtype} of shape {tuple(lab.shape)}")
+        lab = lab.long()
+        if lab.numel() == 0 or int(lab.max()) < 1:
+            raise ValueError("labels has no positive label (0 is background)")
+        if int(lab.min()) < 0:
+            raise ValueError("labels must be >= 0 (0 is background)")
+        vox = torch.nonzero(lab)
+        roi = lab[vox[:, 0], vox[:, 1], vox[:, 2]] - 1
+        n_rois = int(lab.max())
+        count = torch.bincount(roi, minlength=n_rois).double()
+        return cls(roi, vox, 1.0 / count[roi], n_rois, tuple(lab.shape), n_levels, device)
+
+    @property
+    def n_entries(self) -> int:
+        """Table entries the readout kernel walks per batch item: the mean's and every level's coefficients."""
+        return self.n_mean_entries + self.n_coef_entries
+
+
 def denormalize(volume: torch.Tensor, mean_vols, std_vols) -> torch.Tensor:
     """``(vol * 2**len(vol)) * std + mean`` exactly as CWFA.py:1041 writes it (``len`` of a (B,...) tensor = B)."""
     return (volume * 2 ** len(volume)) * std_vols + mean_vols

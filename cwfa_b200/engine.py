@@ -20,7 +20,7 @@ import torch
 
 from . import modules as Fm
 from . import networks, ops, tc
-from .data import LensletLayout
+from .data import LensletLayout, RoiSet
 from .pipeline import CWFAModel, lrnn_mean_volume
 
 
@@ -588,21 +588,28 @@ class CWFAEngine:
         not affine in z; more than 48 detail channels; H * W not a multiple of 4; ``use_f8 = False``) and for a negative
         temperature.  ``sensor``: ``views`` is a raw sensor frame (see ``reconstruct``)."""
         sigma = self._posterior_exact_sigma(temperature)
+        vol, levels = self._scale_pass(views, mean_vols, sensor, _side_streams)
+        std = None                                                # the LRNN volume is deterministic: std 0 (NULL)
+        for hi8, sc8 in levels:
+            vol, std = tc.haar1d_merge_std_f8(vol, std, hi8, sc8, sigma)
+        return vol, std
+
+    def _scale_pass(self, views, mean_vols, sensor, side_streams):
+        """The LRNN volume and, from the top level down (n = L-1 .. 0), every level's z = 0 detail half and scale d hi / d z as
+        ``(hi8, scale8)`` F8 tensors: the LRNN and the levels as independent jobs (parallel branches under graph capture)."""
         L1 = self.model.n_levels
         v8 = self._views_c8(views, sensor)
         mv_last = lrnn_mean_volume(mean_vols, L1)
 
         def level(n):
             lf8 = self._lf(n, v8, None)
-            return self._level_detail_inverse_f8(n, self._trunks(n, lf8), self.levels[n]["f8"], lf8, mean_vols[n], None, with_scale=True)
+            (_, hi8, sc8), _ = self._level_detail_inverse_f8(n, self._trunks(n, lf8), self.levels[n]["f8"], lf8, mean_vols[n], None,
+                                                             with_scale=True)
+            return hi8, sc8
 
         jobs = [lambda: self.lrnn(v8, mv_last)] + [(lambda n=n: level(n)) for n in range(L1 - 1, -1, -1)]
-        results = self._run_jobs(jobs, _side_streams)
-        vol, std = results[0], None                               # the LRNN volume is deterministic: std 0 (NULL)
-        for k in range(L1):
-            (_, hi8, sc8), _ = results[1 + k]
-            vol, std = tc.haar1d_merge_std_f8(vol, std, hi8, sc8, sigma)
-        return vol, std
+        results = self._run_jobs(jobs, side_streams)
+        return results[0], results[1:]
 
     def reconstruct_posterior_exact_graphed(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]],
                                             temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None):
@@ -627,6 +634,74 @@ class CWFAEngine:
             with torch.cuda.graph(graph):
                 out = self.reconstruct_posterior_exact(sv, sm, temperature, sensor=sensor, _side_streams=side)
             g = self._graphs[key] = (graph, sv, sm, out, sensor)    # the graph reads the layout's coordinates: keep it alive
+        graph, sv, sm, out = g[:4]
+        sv.copy_(views, non_blocking=True)
+        for d, s_ in zip(sm, mean_vols):
+            if d is not None:
+                d.copy_(s_, non_blocking=True)
+        graph.replay()
+        return out
+
+    # ---- exact posterior mean and standard deviation of region readouts (neuron traces) ----------------------------------
+    def _roi_check(self, rois: RoiSet, device: torch.device):
+        if not isinstance(rois, RoiSet):
+            raise TypeError(f"rois must be a cwfa_b200.RoiSet, got {type(rois).__name__}")
+        ch0, H, W = self.model.conv_inn[0].global_out_shapes[0]
+        shape = (2 * int(ch0), int(H), int(W))
+        if tuple(rois.volume_shape) != shape or rois.n_levels != self.model.n_levels:
+            raise ValueError(f"the RoiSet is for {tuple(rois.volume_shape)} volumes with {rois.n_levels} levels; this model "
+                             f"reconstructs {shape} volumes with {self.model.n_levels} levels")
+        if rois.device != device:
+            raise ValueError(f"the RoiSet is on {rois.device}, the views on {device}")
+
+    @torch.no_grad()
+    def roi_posterior_exact(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], rois: RoiSet,
+                            temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None, _side_streams=None):
+        """The reconstruction and the exact posterior mean and standard deviation of every readout of ``rois`` (a neuron's
+        trace value: a weighted sum over its footprint), in one inverse pass, for any batch size: ``(volume, roi_mean,
+        roi_std)``, volume (B, D, H, W) bitwise ``reconstruct(views, mean_vols, temperature=0)``, roi_mean and roi_std (B, R) fp32.
+
+        On CAT-only levels level n's detail half is affine in its latent, hi_n[e] = beta_n[e] + alpha_n[e] z_n[pi_n(e)] (alpha_n
+        carried by ``coupling_f8_scale``), the levels are independent and the Haar merges are orthonormal, so for r = sum_v w_v V_v,
+        exactly, E[r] = sum_v w_v V(z = 0)_v and Var[r] = sigma_T^2 sum_n sum_e (alpha_n[e] w~_n[e])^2, w~_n being level n's
+        Haar detail coefficients of the weight volume (``RoiSet``).  This accounts for every covariance between the ROI's voxels:
+        the per-voxel std of ``reconstruct_posterior_exact`` cannot be combined into a readout's std.  sigma_T^2 =
+        ``truncated_normal_var(temperature)`` (default ``cfg.INN_z_temperature``).  Only the mean and std are exact.
+
+        Raises ValueError as ``reconstruct_posterior_exact`` does, and for a RoiSet whose volume shape or level count is not the
+        model's, or which is on another device.  ``sensor``: ``views`` is a raw sensor frame (see ``reconstruct``)."""
+        sigma = self._posterior_exact_sigma(temperature)
+        self._roi_check(rois, views.device)
+        vol, levels = self._scale_pass(views, mean_vols, sensor, _side_streams)
+        for hi8, _ in levels:
+            vol = tc.haar1d_merge_f8(vol, hi8)
+        roi_mean, roi_std = tc.roi_readout_f8(vol, [sc8 for _, sc8 in reversed(levels)], rois, sigma)
+        return vol, roi_mean, roi_std
+
+    def roi_posterior_exact_graphed(self, views: torch.Tensor, mean_vols: Sequence[Optional[torch.Tensor]], rois: RoiSet,
+                                    temperature: Optional[float] = None, sensor: Optional[LensletLayout] = None):
+        """``roi_posterior_exact`` as one CUDA-graph replay, the LRNN and the levels as parallel branches.  A graph per shapes,
+        temperature and RoiSet (the graph reads its tables and keeps it alive).  The returned (volume, roi_mean, roi_std) are the
+        graph's static outputs, overwritten by the next call with the same key."""
+        sigma = self._posterior_exact_sigma(temperature)
+        self._roi_check(rois, views.device)
+        key = ("roi_posterior_exact", tuple(views.shape), tuple(None if m is None else tuple(m.shape) for m in mean_vols),
+               views.device.index, sigma, id(rois), None if sensor is None else (id(sensor), views.dtype))
+        g = self._graphs.get(key)
+        if g is None:
+            sv = views.clone()
+            sm = [None if m is None else m.clone() for m in mean_vols]
+            s = torch.cuda.Stream()
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                for _ in range(2):
+                    self.roi_posterior_exact(sv, sm, rois, temperature, sensor=sensor)
+            torch.cuda.current_stream().wait_stream(s)
+            graph = torch.cuda.CUDAGraph()
+            side = [torch.cuda.Stream() for _ in range(self.model.n_levels + 1)] if self.parallel_branches else None
+            with torch.cuda.graph(graph):
+                out = self.roi_posterior_exact(sv, sm, rois, temperature, sensor=sensor, _side_streams=side)
+            g = self._graphs[key] = (graph, sv, sm, out, rois, sensor)   # the graph reads the tables and the layout: keep them alive
         graph, sv, sm, out = g[:4]
         sv.copy_(views, non_blocking=True)
         for d, s_ in zip(sm, mean_vols):

@@ -613,6 +613,37 @@ def haar1d_merge_std_f8(lo: torch.Tensor, std_lo: Optional[torch.Tensor], hi8: t
     return x, std_x
 
 
+def roi_readout_f8(vol: torch.Tensor, scales8, rois, sigma: float):
+    """Posterior mean and exact standard deviation of the readouts of ``rois`` (``data.RoiSet``) from the z = 0 volume ``vol``
+    (B, D, H, W) and every level's F8 scale tensor ``scales8[n]`` (B, ceil(ch_n / 8), H, W, 8) with ch_n = D / 2^(n+1)
+    (``coupling_f8_scale``): ``(mean, std)``, (B, R) fp32 each, mean = sum_v w_v vol_v and
+    std = sigma sqrt(sum_n sum_e (w~_n[e] scales8[n][e])^2)."""
+    import ctypes as C
+    vol = _ck(vol, "vol")
+    if vol.dim() != 4:
+        raise ValueError(f"roi_readout_f8: vol must be (B, D, H, W), got shape {tuple(vol.shape)}")
+    B, D, H, W = vol.shape
+    L = len(scales8)
+    if (D, H, W) != tuple(rois.volume_shape) or L != rois.n_levels:
+        raise ValueError(f"roi_readout_f8: the RoiSet is for {tuple(rois.volume_shape)} volumes with {rois.n_levels} levels, got "
+                         f"{(D, H, W)} and {L} scale tensors")
+    if rois.device != vol.device:
+        raise ValueError(f"roi_readout_f8: the RoiSet is on {rois.device}, the volume on {vol.device}")
+    for n, s in enumerate(scales8):
+        want = (B, ch8(D >> (n + 1)) // 8, H, W, 8)
+        if tuple(s.shape) != want or s.dtype != torch.float32 or not s.is_contiguous() or s.device != vol.device:
+            raise ValueError(f"roi_readout_f8: scales8[{n}] must be a contiguous fp32 F8 tensor of shape {want} on {vol.device}")
+    R = rois.n_rois
+    mean = torch.empty((B, R), device=vol.device, dtype=torch.float32)
+    std = torch.empty_like(mean)
+    ptrs = (C.c_void_p * L)(*[s.data_ptr() for s in scales8])
+    strides = (C.c_int64 * L)(*[s[0].numel() for s in scales8])
+    _lib.call("cwfa_roi_readout_f8", vol.data_ptr(), D * H * W, ptrs, strides, L, rois.mean_ptr.data_ptr(), rois.mean_idx.data_ptr(),
+              rois.mean_w.data_ptr(), rois.coef_ptr.data_ptr(), rois.coef_idx.data_ptr(), rois.coef_val.data_ptr(), B, R,
+              float(sigma), mean.data_ptr(), std.data_ptr(), _stream())
+    return mean, std
+
+
 def coupling_f8_samples(b: C8, pc: PackedConv, x8: torch.Tensor, samples: int, *, ch: int, clamp: float = 2.0, k_atan: float = 0.636,
                         t_ext8: Optional[torch.Tensor] = None, t_scale: float = 1.0, perm: Optional[torch.Tensor] = None,
                         perm_axis: int = 0, logdet: torch.Tensor = None, accumulate: bool = True,

@@ -335,6 +335,19 @@ int cwfa_coupling_f8_scale(const void* b_c8, const void* w_packed, const float* 
  * Rejected: sigma < 0 or not finite, a NULL lo / hi_f8 / scale_f8 / x / std_x, odd C, P % 4 != 0, unaligned pointers. */
 int cwfa_haar1d_inv_std_f8(const float* lo, const float* std_lo, const float* hi_f8, const float* scale_f8, float sigma, float* x,
                            float* std_x, int B, int C, int64_t P, void* stream);
+/* Posterior mean and exact standard deviation of R region readouts r = sum_v w_v V_v of each of B volumes, when every level's
+ * detail half is hi_n + sigma * scale_n * z_n with independent unit-variance latents (cwfa_coupling_f8_scale):
+ * mean[b, r] = sum_v w_v vol[b, v] and std[b, r] = sigma sqrt(sum_n sum_e (coef_n[e] scale_n[b, e])^2), fp64 sums, written (B, R).
+ * vol: B items of vol_stride floats (the z = 0 volume).  scale_f8, scale_stride: HOST arrays of L device pointers to the F8 scale
+ * tensors and their floats per batch item.  Tables (device, RoiSet in cwfa_b200/data.py): mean_ptr (R + 1) int64 and
+ * (mean_idx, mean_w), a CSR over ROIs of (offset into one volume, weight); coef_ptr (L, R + 1) int64 and (coef_idx, coef_val),
+ * level n's CSR over ROIs of (offset into one item of scale_f8[n], coefficient), offsets into the shared arrays.  One warp per
+ * (b, ROI), no atomics: bitwise reproducible.  Rejected before any device access: L outside 1..8, sigma < 0 or not finite,
+ * R < 1, B < 1, a stride < 1, a NULL pointer (also in scale_f8[0..L-1]). */
+int cwfa_roi_readout_f8(const float* vol, int64_t vol_stride, const float* const* scale_f8, const int64_t* scale_stride, int L,
+                        const int64_t* mean_ptr, const int32_t* mean_idx, const float* mean_w, const int64_t* coef_ptr,
+                        const int32_t* coef_idx, const float* coef_val, int B, int R, float sigma, float* mean, float* std,
+                        void* stream);
 /* Split^-1 + IDWT of K >= 2 latent samples fused with their per-voxel mean and unbiased standard deviation (Welford): the K
  * merged volumes are never written.  lo: K rows (B, C/2, P) or, lo_shared = 1, one row for every sample; hi: K rows in F8
  * (hi_f8 = 1; P % 4 == 0, 16-byte aligned) or NCHW; mean, std: (C, P) each. */
